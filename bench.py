@@ -25,6 +25,10 @@ rank evaluates its own 65,536-instance shard).  Prints ONE JSON line (rank 0).
 
 --impl reference times the reference's own CPU evaluation (oracle/_ref when it was built from the
 reference sources, else the oracle port) on all host cores: same config, all 65,536 instances per step.
+
+--dump-outputs DIR writes the headline's last timed step as DIR/g.npy and DIR/jac.npy (rank 0's shard; both arms):
+fp64 instance-major rows of a fixed sample of DUMP_INSTANCES instances (dump_rows()).  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -52,6 +56,7 @@ CONFIG = {"workload": WORKLOAD, "num_contacts": NC, "env": "Ground", "instances_
           "params": "shared (TestBasic.cpp:64-99 parameter set)", "inputs": "synthetic.ground_batch(65536, 4, seed 1002 + 7919*rank)"}
 L2_BYTES = 126 * 1024 * 1024
 METRIC = "constraint+Jacobian evals/sec (instances/s)"
+DUMP_INSTANCES = 32768  # g + jac of all 65,536 instances are 102 MiB in fp64; half of them stay under 64 MB
 
 
 def algorithmic_bytes_per_instance(n, m, nnz):
@@ -154,6 +159,19 @@ def oracle_problem():
     return op.o
 
 
+def dump_rows():
+    """The instances --dump-outputs writes: a fixed, seeded sample, in index order."""
+    return np.sort(np.random.default_rng(0).choice(N_PER_GPU, DUMP_INSTANCES, replace=False))
+
+
+def dump_outputs(dirname, outputs):
+    """outputs: name -> (N_PER_GPU, k) instance-major array; writes the dump_rows() rows as dirname/<name>.npy in fp64."""
+    os.makedirs(dirname, exist_ok=True)
+    rows = dump_rows()
+    for name, a in outputs.items():
+        np.save(os.path.join(dirname, f"{name}.npy"), np.ascontiguousarray(a[rows], dtype=np.float64))
+
+
 def time_cpu(fn, n_instances, budget_s, max_passes=50):
     """Bounded CPU sample: repeat fn() (one pass over n_instances) until ~budget_s of wall time is spent.  Returns
     (instances/s over all timed passes -- the way --impl reference computes its value --, passes, best-pass instances/s)."""
@@ -202,8 +220,10 @@ def run_reference(args):
         fn()
     t_all = time.perf_counter()
     for _ in range(K):
-        fn()
+        res = fn()
     total = time.perf_counter() - t_all
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"g": res["g"], "jac": res["jac"]})
     value = N_PER_GPU * K / total
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": "instances/s",
             "n_gpus": args.gpus, "steps": K, "warmup": W, "ms_per_step": 1e3 * total / K,
@@ -260,10 +280,11 @@ def run_ours(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    def measure(prob, x_im, lay, ready, regions, use_graph=True, event_pairs=False):
+    def measure(prob, x_im, lay, ready, regions, use_graph=True, event_pairs=False, dump_to=None):
         """W warm-up steps, then `regions` timed regions of EXACTLY K back-to-back g+Jacobian evaluations each (CUDA events on the
         launch stream, barrier + synchronize on both sides, max over ranks per region).  Steps rotate through buffer sets
-        whose total footprint is >> L2.  Returns dict(ms=[per-region ms/step], launches=..., sets=..., launch=..., ev_ms, ev_k)."""
+        whose total footprint is >> L2.  With dump_to, the last timed step's g and jac go through dump_outputs() right after
+        the timed regions.  Returns dict(ms=[per-region ms/step], launches=..., sets=..., launch=..., ev_ms, ev_k)."""
         N = x_im.shape[0]
         n, m, nnz = prob.n, prob.m, prob.nnz
         per_launch = algorithmic_bytes_per_instance(n, m, nnz) * N
@@ -273,9 +294,11 @@ def run_ours(args):
         xs = [base] + [base.clone() for _ in range(sets - 1)]
         gs = [torch.empty(shp(m), dtype=torch.float64, device=dev) for _ in range(sets)]
         js = [torch.empty(shp(nnz), dtype=torch.float64, device=dev) for _ in range(sets)]
+        last = [0]  # buffer set of the latest step issued (or captured into a graph: the last capture is the last replayed step)
 
         def step(i):
             s = i % sets
+            last[0] = s
             prob.eval(xs[s], g=True, jac=True, layout=lay, out={"g": gs[s], "jac": js[s]}, inputs_ready=ready)
 
         for i in range(W):
@@ -326,6 +349,8 @@ def run_ours(args):
             e1.record(stream)
             barrier()
             ms.append(max_over_ranks(e0.elapsed_time(e1)) / K)
+        if dump_to:
+            dump_outputs(dump_to, {k: (b[last[0]] if lay == cpl.INSTANCE_MAJOR else b[last[0]].t()).cpu().numpy() for k, b in (("g", gs), ("jac", js))})
         ev_ms = ev_k = None
         if event_pairs:  # per-launch device time with an event pair around every launch (same stream), separate pass
             prob.timing_begin()
@@ -360,7 +385,7 @@ def run_ours(args):
     x_host = make_inputs(rank)
     ready = not args.no_inputs_ready
     launches0 = prob.launch_count()
-    head = measure(prob, x_host, layout, ready, R, event_pairs=True)
+    head = measure(prob, x_host, layout, ready, R, event_pairs=True, dump_to=args.dump_outputs if rank == 0 else None)
     bytes_per_launch = head["bytes_per_launch"]
     ms_per_step = statistics.median(head["ms"])
     value = world * N / (ms_per_step * 1e-3)
@@ -782,6 +807,7 @@ def main():
                     help="do not tell the evaluator that x is independent of the preceding kernel (CPLB_DEVICE_INPUTS_READY)")
     ap.add_argument("--no-graph", action="store_true", help="issue every timed step as a separate launch instead of CUDA-graph replays")
     ap.add_argument("--cpu-seconds", type=float, default=20.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's g and jac (a fixed sample of instances) to DIR/*.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

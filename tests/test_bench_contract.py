@@ -6,13 +6,28 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
+
+import bench
+from helpers import assert_parity
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def run(*args, timeout=600):
     return subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True, timeout=timeout, cwd=ROOT)
+
+
+def check_dump(d):
+    """--dump-outputs wrote fp64 g and jac of the dump_rows() instances, at most 64 MB, equal to the oracle on the same inputs."""
+    assert sorted(os.listdir(d)) == ["g.npy", "jac.npy"]
+    assert sum(os.path.getsize(os.path.join(d, f)) for f in os.listdir(d)) <= 64_000_000
+    got = {k: np.load(os.path.join(d, f"{k}.npy")) for k in ("g", "jac")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    o = bench.oracle_problem()
+    want = o.eval_batch(bench.make_inputs(0)[bench.dump_rows()], want=("g", "jac"))
+    assert_parity(got, {"g": want["g"], "jac": want["jac"]}, o, "bench --dump-outputs")
 
 
 def test_reference_arm_prints_the_contract_line():
@@ -27,6 +42,23 @@ def test_reference_arm_prints_the_contract_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] in ("reference", "port") and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_reference_arm_dumps_its_last_step(tmp_path):
+    """Without oracle/_ref the reference arm runs the C oracle itself, so this checks the dump's rows, dtype, names and size;
+    the parity of the GPU path's dump is test_product_arm_dumps_its_last_step."""
+    r = run("--impl", "reference", "--steps", "2", "--warmup", "0", "--dump-outputs", str(tmp_path / "out"))
+    assert r.returncode == 0, r.stderr[-2000:]
+    check_dump(tmp_path / "out")
+
+
+@pytest.mark.gpu
+def test_product_arm_dumps_its_last_step(cuda_device, tmp_path):
+    r = run("--steps", "5", "--warmup", "3", "--regions", "1", "--no-cpu", "--dump-outputs", str(tmp_path / "out"))
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][0])
+    assert d["gpu_launches"] == 5 and d["timing"]["timed_regions"]["n"] == 1  # launches one timed region issued
+    check_dump(tmp_path / "out")
 
 
 def test_product_arm_needs_a_gpu():
