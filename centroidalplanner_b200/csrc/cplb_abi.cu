@@ -1397,6 +1397,23 @@ cplb_status cplb_solve_device(cplb_problem* p, int64_t num_instances, const doub
     if (options) o = *options;
     if (!(o.tol > 0.0) || !(o.mu_init > 0.0) || o.max_iter < 0 || o.max_backtracks < 1)
         return fail(CPLB_INVALID_ARGUMENT, "solver options: tol and mu_init must be positive, max_iter >= 0, max_backtracks >= 1");
+    if (cplb::solver::team_block_bytes(p->layout.n, p->layout.m, p->layout.nnz, nullptr) > cplb::solver::kMaxTeamBlockBytes) {
+        // one instance's KKT system must fit one CTA's shared memory: name the largest contact count of this kind that does
+        int limit = 0;
+        for (int k = 1; k <= CPLB_MAX_CONTACTS; k++) {
+            std::vector<std::string> names;
+            for (int c = 0; c < k; c++) names.push_back("c" + std::to_string(c));
+            cplb::Layout L;
+            L.build(names, p->env != CPLB_ENV_NONE, p->env == CPLB_ENV_GROUND);
+            if (cplb::solver::team_block_bytes(L.n, L.m, L.nnz, nullptr) > cplb::solver::kMaxTeamBlockBytes) break;
+            limit = k;
+        }
+        return fail(CPLB_INVALID_ARGUMENT,
+                    "cplb_solve_device: %d contacts need %zu bytes of shared memory per instance, more than the %zu a CTA has; "
+                    "at most %d contacts can be solved with this environment",
+                    (int)p->names.size(), cplb::solver::team_block_bytes(p->layout.n, p->layout.m, p->layout.nnz, nullptr),
+                    cplb::solver::kMaxTeamBlockBytes, limit);
+    }
     cplb_status st = bind_device(p);
     if (st != CPLB_OK) return st;
     DeviceGuard dg(p->device);

@@ -36,26 +36,8 @@ namespace solver {
 struct DeviceTeam {
     int rank, size;
     __device__ __forceinline__ void sync() const { __syncthreads(); }
-    // the first warp of the CTA folds (cplb_solver_core.hpp: arr_sum / arr_nanmax / arr_nanmin); butterfly: every lane gets the result
-    __device__ __forceinline__ int lanes() const { return 32; }
-    __device__ __forceinline__ double lane_sum(double v) const
-    {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        return v;
-    }
-    __device__ __forceinline__ double lane_nanmax(double v) const
-    {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v = nanmax(v, __shfl_xor_sync(0xffffffffu, v, o));
-        return v;
-    }
-    __device__ __forceinline__ double lane_nanmin(double v) const
-    {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v = nanmin(v, __shfl_xor_sync(0xffffffffu, v, o));
-        return v;
-    }
+    // the first warp of the CTA folds (cplb_solver_core.hpp: warp_fold, a __shfl_xor butterfly: every lane gets the result)
+    __device__ __forceinline__ int lanes() const { return kWarp; }
 };
 
 constexpr int kThreads = 128;     // vector phases
@@ -302,6 +284,20 @@ struct DeviceEngine {
 
 static size_t align_up(size_t v) { return (v + 255) & ~(size_t)255; }
 
+size_t team_block_bytes(int n, int m, int nnz, int* mats_in_global)
+{
+    // Four teams per SM are what the registers allow (256 threads x 64): where the full block is too large for that, the dense
+    // Jacobian and the Hessian move to global memory (4 contacts: 71 KB -> 49 KB; 4,096 ground solves 0.0891 -> 0.0868 s); smaller
+    // problems keep them in shared memory (CoMPlanner: 35 KB, and the global round trips would cost 10 %)
+    Scratch probe;
+    double dummy = 0.0;
+    size_t bytes = probe.carve(nullptr, n, m, nnz, true) * sizeof(double);
+    const int global = bytes > kMaxTeamBlockBytes / 4 - 1024 ? 1 : 0;
+    if (global) bytes = probe.carve(nullptr, n, m, nnz, true, &dummy, &dummy) * sizeof(double);
+    if (mats_in_global) *mats_in_global = global;
+    return bytes;
+}
+
 cudaError_t solve_device(const CplbParams& P, int im_kernel, const CplbInstParams* per_instance, const ShapeHost& SH, const Options& O, long long N,
                          const double* x0, double* x_out,
                          int32_t* status, int32_t* iterations, double* cost, double* viol, double* dual, double* lam_out, SolveStats* stats,
@@ -379,17 +375,11 @@ cudaError_t solve_device(const CplbParams& P, int im_kernel, const CplbInstParam
     A.T.out_dual = dual;
 
     Scratch probe;
-    // Four teams per SM are what the registers allow (256 threads x 64): where the full block is too large for that, the dense
-    // Jacobian and the Hessian move to global memory (4 contacts: 71 KB -> 49 KB; 4,096 ground solves 0.0891 -> 0.0868 s); smaller
-    // problems keep them in shared memory (CoMPlanner: 35 KB, and the global round trips would cost 10 %)
-    double dummy = 0.0;
-    size_t smem = probe.carve(nullptr, S.n, S.m, S.nnz, true) * sizeof(double);
-    A.mats_in_global = smem > (227 * 1024) / 4 - 1024 ? 1 : 0;
-    if (A.mats_in_global) smem = probe.carve(nullptr, S.n, S.m, S.nnz, true, &dummy, &dummy) * sizeof(double);
+    const size_t smem = team_block_bytes(S.n, S.m, S.nnz, &A.mats_in_global);
     const size_t smem_small = probe.carve(nullptr, S.n, S.m, S.nnz, false) * sizeof(double);
-    if (smem > 227 * 1024) return cudaErrorInvalidConfiguration;
+    if (smem > kMaxTeamBlockBytes) return cudaErrorInvalidConfiguration;  // (cplb_solve_device refuses such shapes up front)
     for (const void* k : {(const void*)k_round_begin, (const void*)k_kkt, (const void*)k_ls_first, (const void*)k_ls_select, (const void*)k_tail})
-        SOLVER_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        SOLVER_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTeamBlockBytes));
 
     // The tail takes over when the working set fits the GPU in one wave of its CTAs (one per instance; `tail_instances` of the
     // options: < 0 picks SMs x resident CTAs, 0 never).

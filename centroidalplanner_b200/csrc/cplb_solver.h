@@ -10,6 +10,13 @@
 namespace cplb {
 namespace solver {
 
+// Shared memory one CTA of the solver kernels may use (sm_100: 227 KB a block).
+constexpr size_t kMaxTeamBlockBytes = 227 * 1024;
+// Bytes of the full team block (Scratch::carve with the KKT matrix) of an n-variable, m-row problem, as the solve launches it;
+// *mats_in_global (may be NULL) says whether the dense Jacobian and the Hessian go to global memory to keep four teams per SM.
+// A problem whose block exceeds kMaxTeamBlockBytes cannot be solved.
+size_t team_block_bytes(int n, int m, int nnz, int* mats_in_global);
+
 struct Workspace;  // device slabs owned by a problem handle, grown on demand
 void workspace_free(Workspace* w);
 

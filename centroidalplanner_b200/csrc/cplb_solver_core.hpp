@@ -15,6 +15,7 @@
 
 #include <math.h>
 #include <stdint.h>
+#include <string.h>
 
 #include <vector>
 
@@ -82,16 +83,45 @@ struct State {
 };
 
 // A team is the set of threads that carry one instance through a phase.  rank / size / sync() as usual; the first lanes() threads
-// form the team's "first warp", which folds team-shared term arrays with lane_* reductions (every lane gets the result; a fixed
-// tree, so the result does not depend on timing).  On the host a team is one thread.
+// form the team's "first warp", which folds team-shared term arrays with warp_fold (every lane gets the result; a fixed tree, so
+// the result does not depend on timing).  On the host a team is one thread, and warp_fold replays the warp's tree.
 struct HostTeam {
     int rank = 0, size = 1;
     void sync() const {}
     int lanes() const { return 1; }
-    double lane_sum(double v) const { return v; }
-    double lane_nanmax(double v) const { return v; }
-    double lane_nanmin(double v) const { return v; }
 };
+
+constexpr int kWarp = 32;  // lanes of the GPU team's first warp (DeviceTeam::lanes)
+
+// Fold of up to two strided index ranges by the first warp: lane l folds step1 over e = l, l + 32, ... < n1, then step2 over
+// e = l, l + 32, ... < n2, from `init`; the 32 partials combine in the __shfl_xor butterfly v[l] = op(v[l], v[l ^ o]),
+// o = 16, 8, 4, 2, 1.  The host (one thread) computes the same 32 partials and the same tree, so both sides return the same
+// bits, signed zeros included (op's operand order is the device's).
+template <class Team, class Op, class Step1, class Step2>
+CPLB_HD double warp_fold(const Team& team, double init, Op op, int n1, Step1 step1, int n2, Step2 step2)
+{
+#if defined(__CUDA_ARCH__)
+    double v = init;
+    for (int e = team.rank; e < n1; e += kWarp) v = step1(v, e);
+    for (int e = team.rank; e < n2; e += kWarp) v = step2(v, e);
+#pragma unroll
+    for (int o = kWarp / 2; o > 0; o >>= 1) v = op(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+#else
+    (void)team;
+    double v[kWarp], w[kWarp];
+    for (int l = 0; l < kWarp; l++) {
+        v[l] = init;
+        for (int e = l; e < n1; e += kWarp) v[l] = step1(v[l], e);
+        for (int e = l; e < n2; e += kWarp) v[l] = step2(v[l], e);
+    }
+    for (int o = kWarp / 2; o > 0; o >>= 1) {
+        for (int l = 0; l < kWarp; l++) w[l] = op(v[l], v[l ^ o]);
+        for (int l = 0; l < kWarp; l++) v[l] = w[l];
+    }
+    return v[0];
+#endif
+}
 
 CPLB_HD bool finite_d(double v) { return v == v && v - v == 0.0; }
 CPLB_HD double dmax(double a, double b) { return a > b ? a : b; }   // NaN-free callers only (torch.maximum propagates NaN: handled where it matters)
@@ -102,6 +132,71 @@ CPLB_HD double nanmax(double a, double b) { return (a != a) ? a : ((b != b) ? b 
 CPLB_HD double nanmin(double a, double b) { return (a != a) ? a : ((b != b) ? b : (a < b ? a : b)); }
 CPLB_HD double clamp_min(double v, double lo) { return (v != v) ? v : (v < lo ? lo : v); }
 CPLB_HD double clamp_max(double v, double hi) { return (v != v) ? v : (v > hi ? hi : v); }
+
+CPLB_HD uint64_t bits_of(double v)
+{
+#if defined(__CUDA_ARCH__)
+    return (uint64_t)__double_as_longlong(v);
+#else
+    uint64_t u;
+    memcpy(&u, &v, sizeof u);
+    return u;
+#endif
+}
+CPLB_HD double double_of(uint64_t u)
+{
+#if defined(__CUDA_ARCH__)
+    return __longlong_as_double((long long)u);
+#else
+    double v;
+    memcpy(&v, &u, sizeof v);
+    return v;
+#endif
+}
+
+// Natural logarithm from + - * / and exponent manipulation only, so that the GPU (-fmad=false) and the host (-ffp-contract=off)
+// return the same bits; CUDA's and the C library's log are different algorithms, and the barrier terms of the merit function
+// would part the two solves.  fdlibm's __ieee754_log (Sun Microsystems, 1993): x = 2^k (1 + f) with 1 + f in [sqrt(2)/2, sqrt(2)),
+// log(1 + f) = 2 atanh(s), s = f / (2 + f), as a minimax polynomial in s^2, plus k ln2 as a hi/lo pair.  Error < 1 ulp;
+// log(1) = 0, log(+-0) = -inf, log(x < 0) = NaN, log(inf) = inf, NaN -> NaN; subnormals are scaled by 2^54 first.
+CPLB_HD double log_hd(double x)
+{
+    const double ln2_hi = double_of(0x3fe62e42fee00000ull), ln2_lo = double_of(0x3dea39ef35793c76ull);
+    const double Lg1 = double_of(0x3fe5555555555593ull), Lg2 = double_of(0x3fd999999997fa04ull), Lg3 = double_of(0x3fd2492494229359ull),
+                 Lg4 = double_of(0x3fcc71c51d8e78afull), Lg5 = double_of(0x3fc7466496cb03deull), Lg6 = double_of(0x3fc39a09d078c69full),
+                 Lg7 = double_of(0x3fc2f112df3e5244ull);
+    uint64_t u = bits_of(x);
+    int32_t hx = (int32_t)(u >> 32);
+    const uint32_t lx = (uint32_t)u;
+    int k = 0;
+    if (hx < 0x00100000) {                                               // x < 2^-1022
+        if (((hx & 0x7fffffff) | lx) == 0) return double_of(0xfff0000000000000ull);  // log(+-0) = -inf
+        if (hx < 0) return double_of(0x7ff8000000000000ull);               // log(negative) = NaN
+        k -= 54;                                                           // subnormal: scale up
+        x *= 18014398509481984.0;                                          // 2^54
+        u = bits_of(x);
+        hx = (int32_t)(u >> 32);
+    }
+    if (hx >= 0x7ff00000) return x + x;                                    // inf or NaN
+    k += (hx >> 20) - 1023;
+    hx &= 0x000fffff;
+    const int32_t i = (hx + 0x95f64) & 0x100000;                           // mantissa >= sqrt(2): halve it, k + 1
+    x = double_of(((uint64_t)(uint32_t)(hx | (i ^ 0x3ff00000)) << 32) | (u & 0xffffffffull));
+    k += i >> 20;
+    const double f = x - 1.0, dk = (double)k;
+    if ((0x000fffff & (2 + hx)) < 3) {                                     // |f| < 2^-20
+        if (f == 0.0) return k == 0 ? 0.0 : dk * ln2_hi + dk * ln2_lo;
+        const double R = f * f * (0.5 - 0.33333333333333333 * f);
+        return k == 0 ? f - R : dk * ln2_hi - ((R - dk * ln2_lo) - f);
+    }
+    const double s = f / (2.0 + f), z = s * s, w = z * z;
+    const double t1 = w * (Lg2 + w * (Lg4 + w * Lg6)), t2 = z * (Lg1 + w * (Lg3 + w * (Lg5 + w * Lg7))), R = t2 + t1;
+    if (((hx - 0x6147a) | (0x6b851 - hx)) > 0) {
+        const double hfsq = 0.5 * f * f;
+        return k == 0 ? f - (hfsq - s * (hfsq + R)) : dk * ln2_hi - ((hfsq - (s * (hfsq + R) + dk * ln2_lo)) - f);
+    }
+    return k == 0 ? f - s * (f - R) : dk * ln2_hi - ((s * (f - R) - dk * ln2_lo) - f);
+}
 
 // IPOPT's starting-point projection (Waechter & Biegler 2006, section 3.6)
 CPLB_HD double push_inside(double v, double lo, double hi, bool has_lo, bool has_hi, double k1, double k2)
@@ -322,24 +417,32 @@ CPLB_HD double jt_lam(const Inst& I, int j, const double* lam)
 // Folds over team-shared term arrays by the team's first warp (callers: threads with rank < lanes() only, all of them): each lane
 // folds a strided share, the lanes combine in a fixed tree.  One thread doing these alone costs ~100 cycles per element (dependent
 // fp64 compares behind shared-memory loads) -- the serial blocks were a tenth of an iteration's latency.
+struct OpSum {
+    CPLB_HD double operator()(double a, double b) const { return a + b; }
+};
+struct OpNanmax {
+    CPLB_HD double operator()(double a, double b) const { return nanmax(a, b); }
+};
+struct OpNanmin {
+    CPLB_HD double operator()(double a, double b) const { return nanmin(a, b); }
+};
+struct NoStep {
+    CPLB_HD double operator()(double v, int) const { return v; }
+};
 template <class Team>
 CPLB_HD double arr_nanmax(const Team& team, const double* a, int count, double init)
 {
-    for (int e = team.rank; e < count; e += team.lanes()) init = nanmax(init, a[e]);
-    return team.lane_nanmax(init);
+    return warp_fold(team, init, OpNanmax{}, count, [&](double v, int e) { return nanmax(v, a[e]); }, 0, NoStep{});
 }
 template <class Team>
 CPLB_HD double arr_nanmin(const Team& team, const double* a, int count, double init)
 {
-    for (int e = team.rank; e < count; e += team.lanes()) init = nanmin(init, a[e]);
-    return team.lane_nanmin(init);
+    return warp_fold(team, init, OpNanmin{}, count, [&](double v, int e) { return nanmin(v, a[e]); }, 0, NoStep{});
 }
 template <class Team>
 CPLB_HD double arr_sum(const Team& team, const double* a, int count)
 {
-    double acc = 0.0;
-    for (int e = team.rank; e < count; e += team.lanes()) acc += a[e];
-    return team.lane_sum(acc);
+    return warp_fold(team, 0.0, OpSum{}, count, [&](double v, int e) { return v + a[e]; }, 0, NoStep{});
 }
 
 // ---- phase 0a: project the starting point (before the first evaluation) ------------------------------------------------------
@@ -398,6 +501,10 @@ CPLB_HD void phase_init_scale(const Team& team, const Shape& S, const State& T, 
         }
         T.dobj[i] = dmin(O.max_gradient / dmax(gmax, 1e-300), 1.0);
         T.status[i] = bad ? kInvalidNumber : kStatusRunning;
+        if (bad) {  // no round measures a rejected start: its residuals are NaN (include/cpl_batched.h)
+            T.out_viol[i] = double_of(0x7ff8000000000000ull);
+            T.out_dual[i] = double_of(0x7ff8000000000000ull);
+        }
         T.iters[i] = 0;
         T.polish[i] = 0;
         T.active[i] = bad ? 0 : 1;
@@ -484,16 +591,17 @@ CPLB_HD void phase_round_begin(const Team& team, const Shape& S, const State& T,
         const double sd = clamp_min(arr_sum(team, t_sum, nk) / (double)(m + 2 * n + 2 * m), 100.0) / 100.0;
         const double dual = arr_nanmax(team, t_res, nk, 0.0) / sd, prim = arr_nanmax(team, t_prim, m, 0.0);
         auto comp = [&](double mu) {  // max |gap x multiplier - mu| over the bounded components, / sd
-            double e = 0.0;
-            for (int j = team.rank; j < n; j += team.lanes()) {
+            const auto xs = [&](double e, int j) {
                 if (p_xl[j] != -1.0) e = nanmax(e, dabs(p_xl[j] - mu));
                 if (p_xu[j] != -1.0) e = nanmax(e, dabs(p_xu[j] - mu));
-            }
-            for (int r = team.rank; r < m; r += team.lanes()) {
+                return e;
+            };
+            const auto ss = [&](double e, int r) {
                 if (p_sl[r] != -1.0) e = nanmax(e, dabs(p_sl[r] - mu));
                 if (p_su[r] != -1.0) e = nanmax(e, dabs(p_su[r] - mu));
-            }
-            return team.lane_nanmax(e) / sd;
+                return e;
+            };
+            return warp_fold(team, 0.0, OpNanmax{}, n, xs, m, ss) / sd;
         };
         const double E0 = nanmax(nanmax(dual, prim), comp(0.0));
         const double vmax = arr_nanmax(team, t_viol, m, 0.0);
@@ -503,7 +611,7 @@ CPLB_HD void phase_round_begin(const Team& team, const Shape& S, const State& T,
             const double dp0 = nanmax(dual, prim);
             for (int rep = 0; rep < 4; rep++) {
                 const double Emu = nanmax(dp0, comp(mu_next));
-                if (Emu <= 10.0 * mu_next && mu_next > O.tol / 10.0) mu_next = dmax(dmin(0.2 * mu_next, pow(mu_next, 1.5)), O.tol / 10.0);
+                if (Emu <= 10.0 * mu_next && mu_next > O.tol / 10.0) mu_next = dmax(dmin(0.2 * mu_next, mu_next * sqrt(mu_next)), O.tol / 10.0);  // mu^1.5
             }
         }
       if (team.rank == 0) {
@@ -625,7 +733,7 @@ CPLB_HD void phase_kkt(const Team& team, const Shape& S, const State& T, const O
         h[r] = s_h[r];
         D[r] = s_D[r];
     }
-    const double delta_c = 1e-8 * pow(mu, 0.25);
+    const double delta_c = 1e-8 * sqrt(sqrt(mu));  // mu^0.25 (IEEE sqrt: the same bits on both sides, unlike pow)
     double* t_dx = q.term(3, nk);   // candidate step [dx | ds]
     double* t_hdx = q.term(4, nk);  // H dx
 
@@ -746,7 +854,7 @@ CPLB_HD void phase_kkt(const Team& team, const Shape& S, const State& T, const O
         dvxl[j] = a;
         dvxu[j] = b;
         t_ad[j] = ms(vxu[j], b, S.x_hi[j], ms(vxl[j], a, S.x_lo[j], INFINITY));
-        t_lb[j] = (S.x_lo[j] ? log(q.gxl[j]) : 0.0) + (S.x_hi[j] ? log(q.gxu[j]) : 0.0);
+        t_lb[j] = (S.x_lo[j] ? log_hd(q.gxl[j]) : 0.0) + (S.x_hi[j] ? log_hd(q.gxu[j]) : 0.0);
         const double gphi = S.fixed[j] ? 0.0 : (scaled_df(I, j) - (S.x_lo[j] ? mu / q.gxl[j] : 0.0) + (S.x_hi[j] ? mu / q.gxu[j] : 0.0));
         t_dphi[j] = gphi * q.dx[j];
     }
@@ -756,7 +864,7 @@ CPLB_HD void phase_kkt(const Team& team, const Shape& S, const State& T, const O
         dvsl[r] = a;
         dvsu[r] = b;
         t_ad[n + r] = ms(vsu[r], b, S.s_hi[r], ms(vsl[r], a, S.s_lo[r], INFINITY));
-        t_lb[n + r] = (S.s_lo[r] ? log(q.gsl[r]) : 0.0) + (S.s_hi[r] ? log(q.gsu[r]) : 0.0);
+        t_lb[n + r] = (S.s_lo[r] ? log_hd(q.gsl[r]) : 0.0) + (S.s_hi[r] ? log_hd(q.gsu[r]) : 0.0);
         const double gphi = S.is_eq[r] ? 0.0 : (-(S.s_lo[r] ? mu / q.gsl[r] : 0.0) + (S.s_hi[r] ? mu / q.gsu[r] : 0.0));
         t_dphi[n + r] = gphi * q.ds[r];
         t_h1[r] = dabs(s_h[r]);
@@ -885,7 +993,7 @@ CPLB_HD Trial merit_test(const Team& team, const Inst& I, Scratch& q, const doub
     const double mu = T.mu[i], nu = T.nu[i], keep = mu / nu;
     const bool pol = T.pol[i] != 0;
     double *t_lb = q.term(0, nk), *t_viol = q.term(1, nk), *t_bad = q.term(2, nk);
-    for (int j = team.rank; j < n; j += team.size) t_lb[j] = (S.x_lo[j] ? log(X[j] - S.xl[j]) : 0.0) + (S.x_hi[j] ? log(S.xu[j] - X[j]) : 0.0);
+    for (int j = team.rank; j < n; j += team.size) t_lb[j] = (S.x_lo[j] ? log_hd(X[j] - S.xl[j]) : 0.0) + (S.x_hi[j] ? log_hd(S.xu[j] - X[j]) : 0.0);
     for (int r = team.rank; r < m; r += team.size) {
         const double ct = dc[r] * g_raw[r];
         t_bad[r] = finite_d(ct) ? 0.0 : 1.0;
@@ -899,7 +1007,7 @@ CPLB_HD Trial merit_test(const Team& team, const Inst& I, Scratch& q, const doub
             st = (!S.is_eq[r] && inside) ? ct : s[r];
             vr = S.is_eq[r] ? dabs(ct - sl[r]) : ((S.s_hi[r] ? clamp_min(ct - cu_s[r], 0.0) : 0.0) + (S.s_lo[r] ? clamp_min(cl_s[r] - ct, 0.0) : 0.0));
         } else {
-            lbr = (S.s_lo[r] ? log(st - sl[r]) : 0.0) + (S.s_hi[r] ? log(su[r] - st) : 0.0);
+            lbr = (S.s_lo[r] ? log_hd(st - sl[r]) : 0.0) + (S.s_hi[r] ? log_hd(su[r] - st) : 0.0);
             vr = dabs(ct - st);
         }
         t_lb[n + r] = lbr;

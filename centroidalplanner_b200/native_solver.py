@@ -4,6 +4,8 @@ Same algorithm as centroidalplanner_b200/lockstep_solver.py (the interior-point 
 include/cpl_batched.h), but a round is eight kernel launches -- four batched evaluations of the hot path and four solver
 kernels that hold one instance's KKT system in shared memory -- instead of ~1,500 small torch launches and cuBLAS' batched
 LU.  The two drivers agree to the solver tolerances, not bit for bit (different factorisation, different summation orders).
+Its CPU replay (the same per-instance code on the host, the C oracle behind the evaluations) does agree bit for bit on Ground and
+no-environment problems: every result field, in every mode, after any number of iterations.
 The caller side of SURVEY 8(f) rank 1: cpl::CentroidalPlanner::Solve (src/CentroidalPlanner.cpp:22-34) for N instances.
 """
 from __future__ import annotations

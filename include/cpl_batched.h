@@ -366,8 +366,9 @@ typedef struct cplb_solve_outputs {
     int32_t *status;      /* [N]    CPLB_SOLVE_* */
     int32_t *iterations;  /* [N] */
     double *cost;         /* [N]    MinimizeCentroidalVariables::GetCost at x */
-    double *constr_viol;  /* [N]    max violation of the constraint bounds at x */
-    double *dual_inf;     /* [N]    scaled dual infeasibility at x */
+    double *constr_viol;  /* [N]    max violation of the constraint bounds at x; NaN for a start rejected as
+                             CPLB_SOLVE_INVALID_NUMBER before its first iteration (0 iterations) */
+    double *dual_inf;     /* [N]    scaled dual infeasibility at x; NaN for such a rejected start */
     double *lam;          /* [N m]  constraint multipliers, or NULL */
     int32_t *rounds;              /* HOST: lock-step rounds executed, or NULL */
     int64_t *evaluations;         /* HOST: batched evaluations launched, or NULL */
@@ -380,7 +381,10 @@ typedef struct cplb_solve_outputs {
  * i): every instance then solves ITS planning problem -- its own wrench, mass, friction coefficient, references ... -- which is what
  * a sweep over planning scenarios is; the bounds stay the problem's.
  * Synchronises `cuda_stream` (the host reads one counter per round).  Single-device problems only: one solve batch per GPU,
- * instances shard across GPUs by running one batch per device. */
+ * instances shard across GPUs by running one batch per device.
+ * Shape limit: one instance's KKT system lives in one CTA's shared memory (227 KB on sm_100).  A problem whose block would not fit
+ * -- above 10 contacts with an environment, 13 without one -- is refused with CPLB_INVALID_ARGUMENT and a message naming its
+ * contact count and the largest count of its kind that fits. */
 cplb_status cplb_solve_device(cplb_problem *p, int64_t num_instances, const double *x0, const cplb_instance_params *per_instance,
                               const cplb_solver_options *options, const cplb_solve_outputs *out, void *cuda_stream);
 

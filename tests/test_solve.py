@@ -502,6 +502,26 @@ def test_native_round_reports_the_zero_start_as_invalid_number_and_checks_its_ar
     prob, _, _ = product_problem("ground")
     res = cpl.NativeInteriorPoint(max_iter=5).Solve(prob, torch.zeros(3, prob.n, dtype=torch.float64, device=cuda_device))
     assert res.status.tolist() == [INVALID_NUMBER] * 3 and res.rounds == 0
+    # through the ABI with every result buffer pre-filled with a sentinel: a rejected start reports 0 iterations and NaN
+    # residuals (include/cpl_batched.h), whatever the caller's buffers held
+    import ctypes as C
+    from centroidalplanner_b200 import _cabi
+    from centroidalplanner_b200.problem import _check
+
+    N, f64, i32 = 3, torch.float64, torch.int32
+    x0 = torch.zeros(N, prob.n, dtype=f64, device=cuda_device)
+    buf = dict(x=torch.full((N, prob.n), 7.0, dtype=f64, device=cuda_device), status=torch.full((N,), 77, dtype=i32, device=cuda_device),
+               iters=torch.full((N,), 77, dtype=i32, device=cuda_device), cost=torch.full((N,), 7.0, dtype=f64, device=cuda_device),
+               viol=torch.full((N,), 7.0, dtype=f64, device=cuda_device), dual=torch.full((N,), 7.0, dtype=f64, device=cuda_device),
+               lam=torch.full((N, prob.m), 7.0, dtype=f64, device=cuda_device))
+    out = _cabi.SolveOutputs(*(buf[k].data_ptr() for k in ("x", "status", "iters", "cost", "viol", "dual", "lam")), None, None, None, None)
+    opts = cpl.NativeInteriorPoint(max_iter=5).options
+    _check(prob._lib.cplb_solve_device(prob._h, N, x0.data_ptr(), None, C.byref(opts), C.byref(out),
+                                       C.c_void_p(torch.cuda.current_stream(cuda_device).cuda_stream)))
+    torch.cuda.synchronize(cuda_device)
+    assert buf["status"].tolist() == [INVALID_NUMBER] * N and buf["iters"].tolist() == [0] * N
+    assert torch.isnan(buf["viol"]).all() and torch.isnan(buf["dual"]).all()
+    assert not (buf["x"] == 7.0).any() and not (buf["cost"] == 7.0).any() and not (buf["lam"] == 7.0).any()
     with pytest.raises(ValueError, match="device-resident"):
         cpl.NativeInteriorPoint().Solve(prob, torch.zeros(3, prob.n, dtype=torch.float64))
     with pytest.raises(ValueError):
