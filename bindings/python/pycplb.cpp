@@ -169,6 +169,19 @@ PYBIND11_MODULE(pycplb, m)
             return py::make_tuple(c.rounds, c.evaluations, c.instance_evaluations);
         }, py::arg("num_instances"), py::arg("x0"), py::arg("x"), py::arg("status"), py::arg("iterations"), py::arg("cost"),
              py::arg("constr_viol"), py::arg("dual_inf"), py::arg("lam") = 0, py::arg("stream") = 0, py::arg("tol") = 1e-3, py::arg("max_iter") = 500)
+        // first-order derivative test at x (cplb_derivative_test_device); every array argument is a raw device pointer (0 = not wanted)
+        .def("derivative_test_device", [](cplb::BatchedProblem& p, int64_t N, uintptr_t x, uintptr_t num_wrong, uintptr_t num_wrong_outside,
+                                          uintptr_t max_rel_error, uintptr_t worst_row, uintptr_t worst_col, uintptr_t jac_fd, uintptr_t grad_fd,
+                                          uintptr_t stream, double perturbation, double tol) {
+            cplb_derivative_test_options o{perturbation, tol};
+            cplb_derivative_test_outputs out{reinterpret_cast<int32_t*>(num_wrong), reinterpret_cast<int32_t*>(num_wrong_outside),
+                                             reinterpret_cast<double*>(max_rel_error), reinterpret_cast<int32_t*>(worst_row),
+                                             reinterpret_cast<int32_t*>(worst_col), reinterpret_cast<double*>(jac_fd), reinterpret_cast<double*>(grad_fd)};
+            py::gil_scoped_release nogil;
+            p.DerivativeTestDevice(N, reinterpret_cast<const double*>(x), out, reinterpret_cast<void*>(stream), &o);
+        }, py::arg("num_instances"), py::arg("x"), py::arg("num_wrong") = 0, py::arg("num_wrong_outside") = 0, py::arg("max_rel_error") = 0,
+             py::arg("worst_row") = 0, py::arg("worst_col") = 0, py::arg("jac_fd") = 0, py::arg("grad_fd") = 0, py::arg("stream") = 0,
+             py::arg("perturbation") = 1e-8, py::arg("tol") = 1e-4)
         // raw device pointers (e.g. torch.Tensor.data_ptr()), either layout, asynchronous on `stream`
         .def("eval_device", [](cplb::BatchedProblem& p, int64_t N, int layout, int64_t ld, uintptr_t x, uintptr_t g, uintptr_t jac,
                                uintptr_t cost, uintptr_t grad, uintptr_t stream) {

@@ -67,6 +67,17 @@ class SolveOutputs(C.Structure):
                 ("tail_instances", C.POINTER(C.c_int64))]
 
 
+class DerivativeTestOptions(C.Structure):
+    """cplb_derivative_test_options"""
+    _fields_ = [("perturbation", C.c_double), ("tol", C.c_double)]
+
+
+class DerivativeTestOutputs(C.Structure):
+    """cplb_derivative_test_outputs (device pointers; None = not wanted)"""
+    _fields_ = [("num_wrong", C.c_void_p), ("num_wrong_outside", C.c_void_p), ("max_rel_error", C.c_void_p), ("worst_row", C.c_void_p),
+                ("worst_col", C.c_void_p), ("jac_fd", C.c_void_p), ("grad_fd", C.c_void_p)]
+
+
 # name -> (restype, argtypes); every symbol include/cpl_batched.h declares
 PROTOTYPES = {
     "cplb_create": (C.c_int, [C.c_int32, C.POINTER(C.c_char_p), C.c_int, C.c_double, C.c_int32, C.POINTER(C.c_void_p)]),
@@ -125,6 +136,9 @@ PROTOTYPES = {
     "cplb_eval_host_wait": (C.c_int, [C.c_void_p, C.c_int32]),
     "cplb_solver_default_options": (None, [C.POINTER(SolverOptions)]),
     "cplb_solve_device": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.POINTER(InstanceParams), C.POINTER(SolverOptions), C.POINTER(SolveOutputs), C.c_void_p]),
+    "cplb_derivative_test_default_options": (None, [C.POINTER(DerivativeTestOptions)]),
+    "cplb_derivative_test_device": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.POINTER(InstanceParams), C.POINTER(DerivativeTestOptions),
+                                              C.POINTER(DerivativeTestOutputs), C.c_void_p]),
     "cplb_host_alloc": (C.c_int, [C.c_size_t, C.POINTER(C.c_void_p)]),
     "cplb_host_free": (C.c_int, [C.c_void_p]),
     "cplb_set_component_major_kernel": (C.c_int, [C.c_void_p, C.c_int32]),

@@ -467,6 +467,15 @@ public:
         return c;
     }
 
+    // IPOPT's first-order derivative test for N instances at x (cplb_derivative_test_device): what `derivative_test first-order`
+    // checks before every solve of the reference (src/CentroidalPlanner.cpp:26).  Device pointers; any output may be nullptr;
+    // asynchronous on `stream`.
+    void DerivativeTestDevice(int64_t N, const double* x, const cplb_derivative_test_outputs& out, void* stream,
+                              const cplb_derivative_test_options* options = nullptr, const cplb_instance_params* per_instance = nullptr)
+    {
+        check(cplb_derivative_test_device(_p, N, x, per_instance, options, &out, stream));
+    }
+
 private:
     std::vector<std::string> _contact_names;
     env::EnvironmentClass::Ptr _env;

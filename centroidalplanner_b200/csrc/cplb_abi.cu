@@ -16,6 +16,7 @@
 #include <vector>
 
 #include "cpl_batched.h"
+#include "cplb_derivtest.h"
 #include "cplb_kernels.h"
 #include "cplb_layout.hpp"
 #include "cplb_params.h"
@@ -109,6 +110,11 @@ struct cplb_problem {
     // cplb_solve_device: device slabs of the native solve round (grown on demand, freed with the problem)
     std::mutex solver_mu;
     cplb::solver::Workspace* solver_ws = nullptr;
+
+    // cplb_derivative_test_device: structural slot of every dense Jacobian entry (row-major m x n, -1 outside the structure),
+    // uploaded at the first call (the structure never changes after creation)
+    std::mutex derivtest_mu;
+    int32_t* slot_of = nullptr;
 
     int find(const char* name) const
     {
@@ -257,6 +263,10 @@ void cplb_destroy(cplb_problem* p)
     if (p->solver_ws) {
         DeviceGuard dg(p->device >= 0 ? p->device : 0);
         cplb::solver::workspace_free(p->solver_ws);
+    }
+    if (p->slot_of) {
+        DeviceGuard dg(p->device);
+        cudaFree(p->slot_of);
     }
     for (auto& pipe : p->pipes) {
         if (pipe.device < 0 || !pipe.streams_ready) continue;
@@ -1440,6 +1450,78 @@ cplb_status cplb_solve_device(cplb_problem* p, int64_t num_instances, const doub
     if (out->evaluations) *out->evaluations = stats.evaluations;
     if (out->instance_evaluations) *out->instance_evaluations = stats.instance_evaluations;
     if (out->tail_instances) *out->tail_instances = stats.tail_instances;
+    return CPLB_OK;
+}
+
+// ---- first-order derivative test (CentroidalPlanner.cpp:26) -------------------------------------------------------------------
+
+void cplb_derivative_test_default_options(cplb_derivative_test_options* o)
+{
+    if (!o) return;
+    o->perturbation = 1e-8;  // IPOPT's derivative_test_perturbation
+    o->tol = 1e-4;           // derivative_test_tol
+}
+
+// The dense (row, col) -> slot table of the problem on its device, uploaded once.  The copy runs on a stream of its own and is
+// waited for there, so the caller's stream is never synchronised.
+static cplb_status derivtest_slot_table(cplb_problem* p)
+{
+    std::lock_guard<std::mutex> lk(p->derivtest_mu);
+    if (p->slot_of) return CPLB_OK;
+    const cplb::Layout& L = p->layout;
+    std::vector<int32_t> table((size_t)L.m * L.n, -1);
+    for (int s = 0; s < L.nnz; s++) table[(size_t)L.iRow[s] * L.n + L.jCol[s]] = s;
+    const size_t bytes = table.size() * sizeof(int32_t);
+    int32_t* d = nullptr;
+    CPLB_CUDA(cudaMalloc(&d, bytes));
+    cudaStream_t up = nullptr;
+    cudaError_t e = cudaStreamCreateWithFlags(&up, cudaStreamNonBlocking);
+    if (e == cudaSuccess) {
+        e = cudaMemcpyAsync(d, table.data(), bytes, cudaMemcpyHostToDevice, up);
+        const cudaError_t e2 = cudaStreamSynchronize(up);
+        if (e == cudaSuccess) e = e2;
+        cudaStreamDestroy(up);
+    }
+    if (e != cudaSuccess) {
+        cudaFree(d);
+        return cuda_fail(e, "cplb_derivative_test_device: uploading the Jacobian structure");
+    }
+    p->slot_of = d;
+    return CPLB_OK;
+}
+
+cplb_status cplb_derivative_test_device(cplb_problem* p, int64_t num_instances, const double* x, const cplb_instance_params* per_instance,
+                                        const cplb_derivative_test_options* options, const cplb_derivative_test_outputs* out, void* cuda_stream)
+{
+    CPLB_REQUIRE(p);
+    CPLB_REQUIRE(out);
+    if (num_instances < 0) return fail(CPLB_INVALID_ARGUMENT, "num_instances is negative");
+    if (num_instances > 0 && x == nullptr) return fail(CPLB_NULL_POINTER, "x is NULL");
+    cplb_derivative_test_options o;
+    cplb_derivative_test_default_options(&o);
+    if (options) o = *options;
+    if (!(std::isfinite(o.perturbation) && o.perturbation > 0.0))
+        return fail(CPLB_INVALID_ARGUMENT, "derivative test options: perturbation must be finite and positive (got %g)", o.perturbation);
+    if (!(o.tol > 0.0)) return fail(CPLB_INVALID_ARGUMENT, "derivative test options: tol must be positive (got %g)", o.tol);
+    if (p->pipes.size() > 1)
+        return fail(CPLB_INVALID_ARGUMENT, "cplb_derivative_test_device needs a single-device problem (one batch per GPU)");
+    if (num_instances > INT32_MAX) return fail(CPLB_INVALID_ARGUMENT, "num_instances (%lld) must be below 2^31: one CTA per instance", (long long)num_instances);
+    if (num_instances == 0) return CPLB_OK;
+    cplb_status st = bind_device(p);
+    if (st != CPLB_OK) return st;
+    DeviceGuard dg(p->device);
+    if (!dg.ok) return fail(CPLB_CUDA_ERROR, "cudaSetDevice(%d) failed", p->device);
+    st = derivtest_slot_table(p);
+    if (st != CPLB_OK) return st;
+    CplbInstParams q{};
+    const bool per_inst = any_instance_param(per_instance);
+    if (per_inst)
+        for (const auto& f : kInstFields) q.*(f.dst) = per_instance->*(f.src);
+    const cplb::DerivTestOut dout{out->num_wrong, out->num_wrong_outside, out->max_rel_error, out->worst_row, out->worst_col, out->jac_fd, out->grad_fd};
+    cudaError_t e = cplb::launch_derivative_test(p->P, per_inst ? &q : nullptr, x, num_instances, p->slot_of, o.perturbation, o.tol, dout,
+                                                 static_cast<cudaStream_t>(cuda_stream));
+    if (e != cudaSuccess) return cuda_fail(e, "cplb_derivative_test_device");
+    p->launches.fetch_add(1, std::memory_order_relaxed);
     return CPLB_OK;
 }
 

@@ -103,7 +103,7 @@ __device__ __forceinline__ void eval_points_ps(int rank, int size, const CplbPar
     }
 }
 
-__device__ __noinline__ void eval_points(int rank, int size, const CplbParams& P, const CplbInstParams* Q, long long inst, const double* x, int count,
+__device__ __noinline__ inline void eval_points(int rank, int size, const CplbParams& P, const CplbInstParams* Q, long long inst, const double* x, int count,
                                          double* g, double* jac, double* cost, double* grad, unsigned flags)
 {
     if (Q == nullptr) {

@@ -24,14 +24,17 @@ class BatchedCentroidalPlanner:
         self._env = env
         self._cpl_problem = BatchedCplProblem(self._contact_names, robot_mass, env, device=device)
 
-    def Solve(self, x0=None, solver=None, per_instance=None):
+    def Solve(self, x0=None, solver=None, per_instance=None, derivative_test=False):
         """cpl::CentroidalPlanner::Solve (src/CentroidalPlanner.cpp:22-34) for a batch: every row of `x0` (N, n) is one
         instance's starting point (default: one instance at `lockstep_solver.default_start` on the problem's device);
         returns one `Solution` dict per instance (CplProblem::GetSolution, sorted-name order) and keeps the solver's
         report in `last_solve`.  The reference runs ifopt::IpoptSolver here; IPOPT is not part of this repository, so the
         default `solver` is the native lock-step solve round (`NativeInteriorPoint`: same NLP, batched, on the GPU) --
         anything with `Solve(problem, x0, per_instance)` can take its place (e.g. `LockStepInteriorPoint`, the torch driver).  Like the reference, a failed solve is not
-        raised (`:29-32`): inspect `last_solve.status`."""
+        raised (`:29-32`): inspect `last_solve.status`.
+        derivative_test=True first runs the first-order derivative test the reference turns on before every solve (`:26`,
+        BatchedCplProblem.DerivativeTest) at x0 with the same per-instance arrays and keeps its report in `last_derivative_test`;
+        the solve itself is the same either way."""
         import torch
 
         from .lockstep_solver import default_start
@@ -42,6 +45,11 @@ class BatchedCentroidalPlanner:
             if not torch.cuda.is_available():
                 raise RuntimeError("Solve() evaluates on a CUDA device and none is available (there is no CPU evaluation path)")
             x0 = default_start(prob, 1, device=torch.device("cuda", torch.cuda.current_device()))
+        if derivative_test:
+            x0 = torch.as_tensor(x0)
+            if not x0.is_cuda:
+                raise ValueError("the derivative test needs device-resident starting points (there is no CPU evaluation path)")
+            self.last_derivative_test = prob.DerivativeTest(x0.to(torch.float64).contiguous(), per_instance=per_instance)
         self.last_solve = (solver or NativeInteriorPoint()).Solve(prob, x0, per_instance)
         return [prob.GetSolution(xi) for xi in self.last_solve.x.detach().cpu().numpy()]
 

@@ -14,6 +14,7 @@ from __future__ import annotations
 
 import ctypes as C
 import weakref
+from dataclasses import dataclass
 
 import numpy as np
 
@@ -120,6 +121,18 @@ class Superquadric(EnvironmentClass):
         _, r = _v3(self._R)
         _, p = _v3(self._P)
         _check(problem._lib.cplb_set_superquadric(problem._h, c, r, p))
+
+
+@dataclass
+class DerivativeTestReport:
+    """BatchedCplProblem.DerivativeTest: per instance (CUDA tensors, instance-major), see cplb_derivative_test_device."""
+    num_wrong: object          # (N,) int32  wrong entries: gradient + every (row, col) of the dense Jacobian
+    num_wrong_outside: object  # (N,) int32  of those, Jacobian entries outside the declared structure
+    max_rel_error: object      # (N,) float64  rel of the worst entry (NaN stays NaN)
+    worst_row: object          # (N,) int32  -1 = cost gradient
+    worst_col: object          # (N,) int32
+    jac_fd: object             # (N, nnz) float64  forward differences at the structural slots
+    grad_fd: object            # (N, n) float64
 
 
 def _is_torch(t):
@@ -577,6 +590,37 @@ class BatchedCplProblem:
             return ticket.value, res
         _check(self._lib.cplb_eval_host(self._h, C.byref(args)))
         return res
+
+    def DerivativeTest(self, x, per_instance=None, perturbation=1e-8, tol=1e-4, stream=None):
+        """IPOPT's first-order derivative test (the reference turns it on before every solve, src/CentroidalPlanner.cpp:26) for N
+        instances at once: the Jacobian and the cost gradient at x (N, n) -- a contiguous float64 CUDA tensor -- against forward
+        differences of g and f, every entry of the dense Jacobian included.  Asynchronous on the current stream (or `stream`);
+        per_instance: dict of per-instance parameter arrays as for eval().  Returns a DerivativeTestReport."""
+        import torch
+
+        if not (_is_torch(x) and x.is_cuda):
+            raise ValueError("DerivativeTest needs x as a CUDA tensor (there is no CPU evaluation path)")
+        if x.dtype != torch.float64 or not x.is_contiguous() or x.dim() != 2 or x.shape[1] != self.n:
+            raise ValueError(f"x must be a contiguous (N, {self.n}) float64 tensor, got {tuple(x.shape)} {x.dtype}")
+        bound = self.GetDevice()
+        if bound >= 0 and bound != x.device.index:
+            raise ValueError(f"this problem evaluates on cuda:{bound}; x lives on {x.device}")
+        N, dev = x.shape[0], x.device
+        i32, f64 = torch.int32, torch.float64
+        rep = DerivativeTestReport(num_wrong=torch.empty(N, dtype=i32, device=dev), num_wrong_outside=torch.empty(N, dtype=i32, device=dev),
+                                   max_rel_error=torch.empty(N, dtype=f64, device=dev), worst_row=torch.empty(N, dtype=i32, device=dev),
+                                   worst_col=torch.empty(N, dtype=i32, device=dev), jac_fd=torch.empty(N, self.nnz, dtype=f64, device=dev),
+                                   grad_fd=torch.empty(N, self.n, dtype=f64, device=dev))
+        out = _cabi.DerivativeTestOutputs(*[getattr(rep, k).data_ptr() for k in ("num_wrong", "num_wrong_outside", "max_rel_error", "worst_row",
+                                                                                 "worst_col", "jac_fd", "grad_fd")])
+        opt = _cabi.DerivativeTestOptions(float(perturbation), float(tol))
+        pi, keep = self._instance_params(per_instance, N, _cabi.INSTANCE_MAJOR, dev)
+        s = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
+        with torch.cuda.device(dev):
+            _check(self._lib.cplb_derivative_test_device(self._h, N, x.data_ptr(), None if pi is None else C.byref(pi), C.byref(opt),
+                                                         C.byref(out), C.c_void_p(s)))
+        del keep
+        return rep
 
     # the four ifopt::Problem entry points IpoptAdapter calls, batched
     def EvaluateConstraints(self, x, **kw):

@@ -388,6 +388,47 @@ typedef struct cplb_solve_outputs {
 cplb_status cplb_solve_device(cplb_problem *p, int64_t num_instances, const double *x0, const cplb_instance_params *per_instance,
                               const cplb_solver_options *options, const cplb_solve_outputs *out, void *cuda_stream);
 
+/* ---- first-order derivative test ----------------------------------------------------------------------------------------- */
+
+/* Replaces, for N instances at once, the derivative check the reference turns on before every solve: cpl::CentroidalPlanner::Solve
+ * sets IPOPT's `derivative_test first-order` (src/CentroidalPlanner.cpp:26), which compares the Jacobian and the cost gradient with
+ * forward differences of the problem's own g and f at the starting point.  The rule, per instance with x its point:
+ *   h_j  = perturbation * (|x_j| > 1 ? |x_j| : 1)                   (a NaN x_j takes h_j = perturbation)
+ *   fd   = (g(x + h_j e_j) - g(x)) / h_j,  (f(x + h_j e_j) - f(x)) / h_j        (divided by h_j, as IPOPT does)
+ *   rel  = |fd - exact| / (|exact| > 1 ? |exact| : 1)
+ *   an entry is wrong iff !(rel <= tol): NaN and Inf count as wrong.
+ * Every gradient entry and EVERY entry (r, c) of the dense m x n Jacobian is compared; outside the declared structure the exact
+ * value is 0, so a derivative the structure misses is found too.  g, f, the Jacobian and the gradient are the batched evaluator's
+ * own values, bit for bit what cplb_eval_device returns.  The worst entry is the first one with the largest rel (NaN counted as
+ * +inf) in the order: gradient columns 0..n-1, then the Jacobian row by row, column ascending.  One CTA per instance evaluates
+ * the n perturbed points in chunks inside shared memory (csrc/cplb_derivtest.cu); nothing is widened in global memory. */
+typedef struct cplb_derivative_test_options {
+    double perturbation; /* 1e-8: IPOPT's derivative_test_perturbation */
+    double tol;          /* 1e-4: IPOPT's derivative_test_tol */
+} cplb_derivative_test_options;
+void cplb_derivative_test_default_options(cplb_derivative_test_options *options);
+
+typedef struct cplb_derivative_test_outputs { /* DEVICE arrays, instance-major; every pointer may be NULL */
+    int32_t *num_wrong;         /* [N]     wrong entries: gradient + every (row, col) of the dense Jacobian */
+    int32_t *num_wrong_outside; /* [N]     of those, Jacobian entries outside the declared structure */
+    double *max_rel_error;      /* [N]     rel of the worst entry, as computed (NaN stays NaN) */
+    int32_t *worst_row;         /* [N]     -1 = cost gradient */
+    int32_t *worst_col;         /* [N] */
+    double *jac_fd;             /* [N nnz] forward differences at the structural slots, in slot order */
+    double *grad_fd;            /* [N n] */
+} cplb_derivative_test_outputs;
+
+/* x [N n]: the points (DEVICE pointer; the caller's column order).  per_instance: NULL, or per-instance parameter arrays as for
+ * cplb_solve_device (DEVICE pointers, instance-major).  options: NULL = defaults.  Asynchronous on `cuda_stream`, like
+ * cplb_eval_device: it does not synchronise the stream (the first call on a problem uploads a table of the Jacobian structure
+ * once, on a stream of its own).  Counts one launch in cplb_get_launch_count.  Argument errors are reported before any CUDA call:
+ * NULL p or out, or NULL x with N > 0 -> CPLB_NULL_POINTER; N < 0, a perturbation that is not finite and positive, a tol that is
+ * not positive -> CPLB_INVALID_ARGUMENT; N = 0 -> CPLB_OK, nothing launched.  Single-device problems only, like
+ * cplb_solve_device.  Every shape up to CPLB_MAX_CONTACTS contacts is supported, in every environment. */
+cplb_status cplb_derivative_test_device(cplb_problem *p, int64_t num_instances, const double *x, const cplb_instance_params *per_instance,
+                                        const cplb_derivative_test_options *options, const cplb_derivative_test_outputs *out,
+                                        void *cuda_stream);
+
 /* Pinned host memory for cplb_eval_host buffers (cudaHostAlloc / cudaFreeHost). */
 cplb_status cplb_host_alloc(size_t bytes, void **out);
 cplb_status cplb_host_free(void *ptr);
