@@ -27,13 +27,14 @@ dp = C.POINTER(C.c_double)
 ip = C.POINTER(C.c_int32)
 
 
-INSTANCE_PARAM_FIELDS = ("mass", "wrench", "mu", "force_threshold", "ground_z", "com_ref", "com_weight", "pos_ref", "force_ref",
-                         "pos_weight", "force_weight")
+# cplb_instance_params in member order: (name, fixed length, length per contact); doubles per instance = fixed + per_contact * nc
+INSTANCE_PARAMS = (("mass", 1, 0), ("wrench", 6, 0), ("mu", 1, 0), ("force_threshold", 0, 1), ("ground_z", 1, 0), ("com_ref", 3, 0),
+                   ("com_weight", 1, 0), ("pos_ref", 0, 3), ("force_ref", 0, 3), ("pos_weight", 0, 1), ("force_weight", 0, 1))
 
 
 class InstanceParams(C.Structure):
     """cplb_instance_params: optional per-instance parameter arrays (NULL = the problem's shared value)."""
-    _fields_ = [(name, C.c_void_p) for name in INSTANCE_PARAM_FIELDS]
+    _fields_ = [(name, C.c_void_p) for name, _, _ in INSTANCE_PARAMS]
 
 
 class EvalArgs(C.Structure):

@@ -7,6 +7,7 @@
 #include <atomic>
 #include <cmath>
 #include <cstdarg>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <mutex>
@@ -814,34 +815,28 @@ static cplb_status check_args(const cplb_problem* p, const cplb_eval_args* a, un
     return CPLB_OK;
 }
 
-// the per-instance arrays, in one table: ABI field, device-struct field, elements per instance
-using AbiField = const double* cplb_instance_params::*;
-using DevField = const double* CplbInstParams::*;
-struct InstField {
-    AbiField src;
-    DevField dst;
-    int len_fixed, len_per_contact;
-    int len(int nc) const { return len_fixed + len_per_contact * nc; }
-};
-static const InstField kInstFields[] = {
-    {&cplb_instance_params::mass, &CplbInstParams::mass, 1, 0},
-    {&cplb_instance_params::wrench, &CplbInstParams::wrench, 6, 0},
-    {&cplb_instance_params::mu, &CplbInstParams::mu, 1, 0},
-    {&cplb_instance_params::force_threshold, &CplbInstParams::F_thr, 0, 1},
-    {&cplb_instance_params::ground_z, &CplbInstParams::ground_z, 1, 0},
-    {&cplb_instance_params::com_ref, &CplbInstParams::com_ref, 3, 0},
-    {&cplb_instance_params::com_weight, &CplbInstParams::W_com, 1, 0},
-    {&cplb_instance_params::pos_ref, &CplbInstParams::p_ref, 0, 3},
-    {&cplb_instance_params::force_ref, &CplbInstParams::F_ref, 0, 3},
-    {&cplb_instance_params::pos_weight, &CplbInstParams::W_p, 0, 1},
-    {&cplb_instance_params::force_weight, &CplbInstParams::W_F, 0, 1},
-};
+// cplb_instance_params holds the same pointers as CplbInstParams::arr, member i being array i of CplbInstArray
+constexpr size_t inst_array_offset(int a) { return offsetof(CplbInstParams, arr) + a * sizeof(const double*); }
+static_assert(sizeof(cplb_instance_params) == sizeof(CplbInstParams), "cplb_instance_params and CplbInstParams differ in size");
+static_assert(offsetof(cplb_instance_params, mass) == inst_array_offset(CPLB_IA_MASS), "mass");
+static_assert(offsetof(cplb_instance_params, wrench) == inst_array_offset(CPLB_IA_WRENCH), "wrench");
+static_assert(offsetof(cplb_instance_params, mu) == inst_array_offset(CPLB_IA_MU), "mu");
+static_assert(offsetof(cplb_instance_params, force_threshold) == inst_array_offset(CPLB_IA_F_THR), "force_threshold");
+static_assert(offsetof(cplb_instance_params, ground_z) == inst_array_offset(CPLB_IA_GROUND_Z), "ground_z");
+static_assert(offsetof(cplb_instance_params, com_ref) == inst_array_offset(CPLB_IA_COM_REF), "com_ref");
+static_assert(offsetof(cplb_instance_params, com_weight) == inst_array_offset(CPLB_IA_W_COM), "com_weight");
+static_assert(offsetof(cplb_instance_params, pos_ref) == inst_array_offset(CPLB_IA_P_REF), "pos_ref");
+static_assert(offsetof(cplb_instance_params, force_ref) == inst_array_offset(CPLB_IA_F_REF), "force_ref");
+static_assert(offsetof(cplb_instance_params, pos_weight) == inst_array_offset(CPLB_IA_W_P), "pos_weight");
+static_assert(offsetof(cplb_instance_params, force_weight) == inst_array_offset(CPLB_IA_W_F), "force_weight");
 
-static bool any_instance_param(const cplb_instance_params* q)
+// The caller's per-instance arrays (abi may be NULL) as CplbInstParams; false when none is set.
+static bool instance_arrays(const cplb_instance_params* abi, CplbInstParams* q)
 {
-    if (!q) return false;
-    for (const auto& f : kInstFields)
-        if (q->*(f.src)) return true;
+    *q = CplbInstParams{};
+    if (abi) std::memcpy(q, abi, sizeof *q);
+    for (const double* a : q->arr)
+        if (a) return true;
     return false;
 }
 
@@ -873,10 +868,8 @@ static cplb_status eval_device_on(cplb_problem* p, int device, const cplb_eval_a
         CPLB_CUDA(cudaEventCreate(&e1));
         CPLB_CUDA(cudaEventRecord(e0, stream));
     }
-    CplbInstParams q{};
-    const bool per_inst = any_instance_param(args->per_instance);
-    if (per_inst)
-        for (const auto& f : kInstFields) q.*(f.dst) = args->per_instance->*(f.src);
+    CplbInstParams q;
+    const bool per_inst = instance_arrays(args->per_instance, &q);
     if (args->host_flags & CPLB_DEVICE_INPUTS_READY) flags |= CPLB_INPUTS_READY;
     cplb_status st = launch(p, io, args->layout, flags, stream, per_inst ? &q : nullptr);
     if (timed) {
@@ -1002,21 +995,23 @@ struct HostInput {  // one host input array (x or a per-instance parameter array
     const double* user;
     int len;
     size_t off;  // offset (doubles) inside a staging buffer
-    DevField dst;  // nullptr for x
+    int arr;     // CplbInstArray; -1 for x
 };
 
 // x and every per-instance array that is present, laid out after the output sections of a staging buffer
 static std::vector<HostInput> host_inputs(const cplb_problem* p, const cplb_eval_args* args, long long chunk, size_t first_free, size_t* end)
 {
     std::vector<HostInput> in;
-    in.push_back(HostInput{args->x, p->layout.n, 0, nullptr});
+    in.push_back(HostInput{args->x, p->layout.n, 0, -1});
     size_t off = first_free;
-    if (args->per_instance)
-        for (const auto& f : kInstFields)
-            if (args->per_instance->*(f.src)) {
-                in.push_back(HostInput{args->per_instance->*(f.src), f.len(p->layout.nc), off, f.dst});
-                off += (size_t)f.len(p->layout.nc) * chunk;
-            }
+    CplbInstParams user;
+    instance_arrays(args->per_instance, &user);
+    for (int a = 0; a < CPLB_NUM_INST_ARRAYS; a++)
+        if (user.arr[a]) {
+            const int len = cplb_inst_len(a, p->layout.nc);
+            in.push_back(HostInput{user.arr[a], len, off, a});
+            off += (size_t)len * chunk;
+        }
     *end = off;
     return in;
 }
@@ -1089,7 +1084,7 @@ static cplb_status eval_host_bounced(cplb_problem* p, HostPipe& pipe, const cplb
             else std::memcpy(hb, in.user + i0 * in.len, (size_t)cnt * in.len * sizeof(double));
             cudaError_t e = cudaMemcpyAsync(d + in.off, hb, (size_t)in.len * chunk * sizeof(double), cudaMemcpyHostToDevice, stream);
             if (e != cudaSuccess) return bail(cuda_fail(e, "cudaMemcpyAsync (host to device)"));
-            if (in.dst) q.*(in.dst) = d + in.off;
+            if (in.arr >= 0) q.arr[in.arr] = d + in.off;
         }
         CplbIo io{d + ox, (flags & CPLB_WANT_G) ? d + og : nullptr, (flags & CPLB_WANT_J) ? d + oj : nullptr,
                   (flags & CPLB_WANT_COST) ? d + oc : nullptr, (flags & CPLB_WANT_GRAD) ? d + ogr : nullptr, chunk, cnt};
@@ -1127,8 +1122,8 @@ static cplb_status enqueue_chunk(cplb_problem* p, HostPipe& pipe, int s, const c
     if (flags & CPLB_WANT_GRAD) { dgr = d; d += (size_t)n * chunk; }
     if (flags & CPLB_WANT_COST) { dc = d; d += (size_t)chunk; }
     // device-side chunk buffers use pitch `chunk` (component-major) or are dense (instance-major)
-    CplbInstParams q{};
-    bool per_inst = false;
+    CplbInstParams user, q{};
+    const bool per_inst = instance_arrays(args->per_instance, &user);
     auto h2d = [&](double* dst, const double* src, int len) -> cplb_status {
         if (cm) CPLB_CUDA(cudaMemcpy2DAsync(dst, chunk * sizeof(double), src + i0, ld * sizeof(double), cnt * sizeof(double), len, cudaMemcpyHostToDevice, stream));
         else CPLB_CUDA(cudaMemcpyAsync(dst, src + i0 * len, (size_t)cnt * len * sizeof(double), cudaMemcpyHostToDevice, stream));
@@ -1136,16 +1131,14 @@ static cplb_status enqueue_chunk(cplb_problem* p, HostPipe& pipe, int s, const c
     };
     cplb_status st = h2d(dx, args->x, n);
     if (st != CPLB_OK) return st;
-    if (args->per_instance)
-        for (const auto& f : kInstFields)
-            if (const double* src = args->per_instance->*(f.src)) {
-                const int len = f.len(p->layout.nc);
-                st = h2d(d, src, len);
-                if (st != CPLB_OK) return st;
-                q.*(f.dst) = d;
-                d += (size_t)len * chunk;
-                per_inst = true;
-            }
+    for (int a = 0; a < CPLB_NUM_INST_ARRAYS; a++)
+        if (user.arr[a]) {
+            const int len = cplb_inst_len(a, p->layout.nc);
+            st = h2d(d, user.arr[a], len);
+            if (st != CPLB_OK) return st;
+            q.arr[a] = d;
+            d += (size_t)len * chunk;
+        }
     CplbIo io{dx, dg_, dj, dc, dgr, chunk, cnt};
     st = launch(p, io, args->layout, flags, stream, per_inst ? &q : nullptr);
     if (st != CPLB_OK) return st;
@@ -1213,9 +1206,10 @@ static cplb_status eval_host_impl(cplb_problem* p, const cplb_eval_args* args, i
     if (flags & CPLB_WANT_J) per_inst += nnz;
     if (flags & CPLB_WANT_COST) per_inst += 1;
     if (flags & CPLB_WANT_GRAD) per_inst += n;
-    if (args->per_instance)
-        for (const auto& f : kInstFields)
-            if (args->per_instance->*(f.src)) per_inst += f.len(p->layout.nc);
+    CplbInstParams user;
+    instance_arrays(args->per_instance, &user);
+    for (int a = 0; a < CPLB_NUM_INST_ARRAYS; a++)
+        if (user.arr[a]) per_inst += cplb_inst_len(a, p->layout.nc);
     const size_t stage_bytes = per_inst * (size_t)chunk * sizeof(double);
     auto set_device = [&](int sh) -> cplb_status {
         if (shards > 1) CPLB_CUDA(cudaSetDevice(p->pipes[(size_t)sh].device));
@@ -1231,8 +1225,7 @@ static cplb_status eval_host_impl(cplb_problem* p, const cplb_eval_args* args, i
     }
 
     bool all_pinned = is_pinned(args->x) && is_pinned(args->g) && is_pinned(args->jac) && is_pinned(args->cost) && is_pinned(args->grad);
-    if (args->per_instance)
-        for (const auto& f : kInstFields) all_pinned = all_pinned && is_pinned(args->per_instance->*(f.src));
+    for (const double* a : user.arr) all_pinned = all_pinned && is_pinned(a);
     if (!all_pinned) {
         if (ticket) return fail(CPLB_INVALID_ARGUMENT, "cplb_eval_host_begin needs pinned host buffers (cplb_host_alloc)");
         if (shards == 1) return eval_host_bounced(p, p->pipes[0], args, flags, ld, chunk, stage_bytes, 0, N);
@@ -1438,10 +1431,8 @@ cplb_status cplb_solve_device(cplb_problem* p, int64_t num_instances, const doub
                                   o.bound_relax_factor, o.max_iter, o.max_backtracks, o.tail_instances};
     cplb::solver::SolveStats stats;
     const long long launches_per_round = 8;
-    CplbInstParams q{};
-    const bool per_inst = any_instance_param(per_instance);
-    if (per_inst)
-        for (const auto& f : kInstFields) q.*(f.dst) = per_instance->*(f.src);
+    CplbInstParams q;
+    const bool per_inst = instance_arrays(per_instance, &q);
     cudaError_t e = cplb::solver::solve_device(p->P, p->im_kernel, per_inst ? &q : nullptr, SH, O, num_instances, x0, out->x, out->status, out->iterations, out->cost,
                                                out->constr_viol, out->dual_inf, out->lam, &stats, &p->solver_ws, static_cast<cudaStream_t>(cuda_stream));
     if (e != cudaSuccess) return cuda_fail(e, "cplb_solve_device");
@@ -1513,10 +1504,8 @@ cplb_status cplb_derivative_test_device(cplb_problem* p, int64_t num_instances, 
     if (!dg.ok) return fail(CPLB_CUDA_ERROR, "cudaSetDevice(%d) failed", p->device);
     st = derivtest_slot_table(p);
     if (st != CPLB_OK) return st;
-    CplbInstParams q{};
-    const bool per_inst = any_instance_param(per_instance);
-    if (per_inst)
-        for (const auto& f : kInstFields) q.*(f.dst) = per_instance->*(f.src);
+    CplbInstParams q;
+    const bool per_inst = instance_arrays(per_instance, &q);
     const cplb::DerivTestOut dout{out->num_wrong, out->num_wrong_outside, out->max_rel_error, out->worst_row, out->worst_col, out->jac_fd, out->grad_fd};
     cudaError_t e = cplb::launch_derivative_test(p->P, per_inst ? &q : nullptr, x, num_instances, p->slot_of, o.perturbation, o.tol, dout,
                                                  static_cast<cudaStream_t>(cuda_stream));

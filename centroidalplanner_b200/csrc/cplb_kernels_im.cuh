@@ -133,8 +133,9 @@ __global__ void __launch_bounds__(WARPS * 32) eval_instance_major(const __grid_c
     const uint32_t xbytes = (uint32_t)(T * n * sizeof(double));
     // bulk copies need 16-byte aligned addresses and sizes: full tiles of 16B-aligned buffers only
     auto is_bulk = [&](long long t) { return aligned16 && (t + 1) * T <= io.N; };
-    const double* const parr[CPLB_NUM_INST_ARRAYS] = {Q.mass, Q.wrench, Q.mu, Q.F_thr, Q.ground_z, Q.com_ref, Q.W_com,
-                                                       Q.p_ref, Q.F_ref, Q.W_p, Q.W_F};
+    // a local copy: reading Q.arr in place changes the generated code of the per-instance variants
+    const double* parr[CPLB_NUM_INST_ARRAYS];
+    for (int a = 0; a < CPLB_NUM_INST_ARRAYS; a++) parr[a] = Q.arr[a];
     // one elected lane: x tile + every staged parameter slice of tile t into buffer `buf`, all on one mbarrier
     auto issue_loads = [&](long long t, int buf) {
         mbar_expect_tx(&bar[buf], xbytes + (uint32_t)(ptot * sizeof(double)));
@@ -353,12 +354,9 @@ cudaError_t launch_im_kernel(const CplbParams& P, const CplbIo& io, unsigned fla
     const unsigned blocks = (unsigned)(want < resident ? want : resident);
     auto al16 = [](const void* p) { return p == nullptr || (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
     int aligned16 = al16(io.x) && al16(io.g) && al16(io.jac) && al16(io.grad) && (T % 2 == 0);
-    if (Q) {
-        const double* const parr[CPLB_NUM_INST_ARRAYS] = {Q->mass, Q->wrench, Q->mu, Q->F_thr, Q->ground_z, Q->com_ref, Q->W_com,
-                                                           Q->p_ref, Q->F_ref, Q->W_p, Q->W_F};
+    if (Q)
         for (int a = 0; a < CPLB_NUM_INST_ARRAYS; a++)
-            if (PT.off[a] >= 0) aligned16 = aligned16 && al16(parr[a]);
-    }
+            if (PT.off[a] >= 0) aligned16 = aligned16 && al16(Q->arr[a]);
     return launch_pdl(kern, blocks, WARPS * 32, smem, st, P, io, flags, aligned16, Q ? *Q : kNoInstParams, PT);
 }
 
@@ -366,15 +364,11 @@ cudaError_t launch_im_kernel(const CplbParams& P, const CplbIo& io, unsigned fla
 inline CplbParamTile make_param_tile(const CplbParams& P, const CplbInstParams* Q, unsigned flags, int T)
 {
     CplbParamTile PT = {};
-    const int nc = P.nc;
-    const int lens[CPLB_NUM_INST_ARRAYS] = {1, 6, 1, nc, 1, 3, 1, 3 * nc, 3 * nc, nc, nc};
     for (int a = 0; a < CPLB_NUM_INST_ARRAYS; a++) {
         PT.off[a] = -1;
-        PT.len[a] = lens[a];
+        PT.len[a] = cplb_inst_len(a, P.nc);
     }
     if (!Q) return PT;
-    const double* const parr[CPLB_NUM_INST_ARRAYS] = {Q->mass, Q->wrench, Q->mu, Q->F_thr, Q->ground_z, Q->com_ref, Q->W_com,
-                                                       Q->p_ref, Q->F_ref, Q->W_p, Q->W_F};
     // Staged for constraint-only evaluations: what the constraint rows read (9 + nc doubles per instance; measured 55 -> 61 %
     // of the roofline at 65,536 x 4 contacts, 69 -> 75 % at 1,048,576).  With the cost or the gradient requested nothing is
     // staged and every array is read with read-only global loads as before: that variant is bound by the cost lane's
@@ -383,13 +377,11 @@ inline CplbParamTile make_param_tile(const CplbParams& P, const CplbInstParams* 
     // Ground problems only: without an environment the extra 1.5 KB per warp costs a resident CTA (59 vs 53 KB: 70 -> 62 % at
     // 1,048,576 x 4 contacts) and the Superquadric rows are bound by their arithmetic (48 vs 45 %, 51 vs 52 %).
     if (flags & (CPLB_WANT_COST | CPLB_WANT_GRAD)) return PT;
-    if (P.env != CPLB_ENV_GROUND_K) return PT;
-    const bool GJ = flags & (CPLB_WANT_G | CPLB_WANT_J), C = false;
-    const bool need[CPLB_NUM_INST_ARRAYS] = {GJ, GJ, GJ, GJ, GJ && P.env == CPLB_ENV_GROUND_K, C, C, C, C, C, C};
-    for (int a = 0; a < CPLB_NUM_INST_ARRAYS; a++)
-        if (parr[a] && need[a]) {
+    if (P.env != CPLB_ENV_GROUND_K || !(flags & (CPLB_WANT_G | CPLB_WANT_J))) return PT;
+    for (int a = 0; a < CPLB_IA_COM_REF; a++)
+        if (Q->arr[a]) {
             PT.off[a] = PT.total;
-            PT.total += T * lens[a];
+            PT.total += T * PT.len[a];
         }
     return PT;
 }

@@ -52,27 +52,46 @@ struct CplbParams {
     double W_F[CPLB_KMAX_CONTACTS];
 };
 
-// Optional per-instance parameter arrays (device memory; NULL = use the shared value of CplbParams), see
-// cplb_instance_params in include/cpl_batched.h.  Same layout rule as x: element e of instance i is arr[i*len + e]
-// (instance-major) or arr[e*ld + i] (component-major); len = 1, 6, nc, 3, 3*nc as noted.
+// The optional per-instance parameter arrays, in the member order of cplb_instance_params (include/cpl_batched.h;
+// cplb_abi.cu pins the correspondence).  The arrays before CPLB_IA_COM_REF are the ones the constraint rows read; the
+// rest only the cost and its gradient.
+enum CplbInstArray {
+    CPLB_IA_MASS,
+    CPLB_IA_WRENCH,
+    CPLB_IA_MU,
+    CPLB_IA_F_THR,     // contact index = position in the caller's name vector
+    CPLB_IA_GROUND_Z,
+    CPLB_IA_COM_REF,
+    CPLB_IA_W_COM,
+    CPLB_IA_P_REF,     // x,y,z of contact 0, then contact 1, ...
+    CPLB_IA_F_REF,
+    CPLB_IA_W_P,
+    CPLB_IA_W_F,
+    CPLB_NUM_INST_ARRAYS
+};
+
+// doubles per instance of array a
+__host__ __device__ constexpr int cplb_inst_len(int a, int nc)
+{
+    switch (a) {
+    case CPLB_IA_WRENCH: return 6;
+    case CPLB_IA_COM_REF: return 3;
+    case CPLB_IA_F_THR: case CPLB_IA_W_P: case CPLB_IA_W_F: return nc;
+    case CPLB_IA_P_REF: case CPLB_IA_F_REF: return 3 * nc;
+    default: return 1;
+    }
+}
+
+// The per-instance arrays of one call (device memory; NULL = use the shared value of CplbParams), indexed by CplbInstArray.
+// Same layout rule as x: element e of instance i is arr[a][i*len + e] (instance-major) or arr[a][e*ld + i] (component-major),
+// len = cplb_inst_len(a, nc).
 struct CplbInstParams {
-    const double* mass;      // 1
-    const double* wrench;    // 6
-    const double* mu;        // 1
-    const double* F_thr;     // nc   (contact index = position in the caller's name vector)
-    const double* ground_z;  // 1
-    const double* com_ref;   // 3
-    const double* W_com;     // 1
-    const double* p_ref;     // 3*nc (x,y,z of contact 0, then contact 1, ...)
-    const double* F_ref;     // 3*nc
-    const double* W_p;       // nc
-    const double* W_F;       // nc
+    const double* arr[CPLB_NUM_INST_ARRAYS];
 };
 
 // Instance-major kernel, per-instance parameter mode: where each staged parameter array's slice of a warp tile sits in the
 // shared-memory parameter buffer (doubles from the buffer start; -1 = not staged: absent, or not needed by the requested
-// outputs).  Array order = the member order of CplbInstParams.
-#define CPLB_NUM_INST_ARRAYS 11
+// outputs), indexed by CplbInstArray.
 struct CplbParamTile {
     int off[CPLB_NUM_INST_ARRAYS];
     int len[CPLB_NUM_INST_ARRAYS];  // doubles per instance of each array

@@ -395,16 +395,15 @@ cudaError_t solve_device(const CplbParams& P, int im_kernel, const CplbInstParam
     ParamGather G{};
     CplbInstParams Q_one{}, Q_fd{}, Q_ls{};
     if (per_instance) {
-        const double* const src[CPLB_NUM_INST_ARRAYS] = {per_instance->mass, per_instance->wrench, per_instance->mu, per_instance->F_thr,
-                                                         per_instance->ground_z, per_instance->com_ref, per_instance->W_com, per_instance->p_ref,
-                                                         per_instance->F_ref, per_instance->W_p, per_instance->W_F};
-        const int nc = P.nc, len[CPLB_NUM_INST_ARRAYS] = {1, 6, 1, nc, 1, 3, 1, 3 * nc, 3 * nc, nc, nc};
         G.reps_fd = S.nf + 1;
         G.reps_ls = kCandidates;
         const size_t rows = 1 + (size_t)G.reps_fd + (size_t)G.reps_ls;
         size_t param_bytes = 0;
-        for (int a = 0; a < CPLB_NUM_INST_ARRAYS; a++)
-            if (src[a]) param_bytes += 3 * 256 + rows * (size_t)len[a] * (size_t)N * sizeof(double);
+        for (int a = 0; a < CPLB_NUM_INST_ARRAYS; a++) {
+            G.src[a] = per_instance->arr[a];
+            G.len[a] = cplb_inst_len(a, P.nc);
+            if (G.src[a]) param_bytes += 3 * 256 + rows * (size_t)G.len[a] * (size_t)N * sizeof(double);
+        }
         if (param_bytes > W->param_bytes) {
             if (W->param_slab) SOLVER_CUDA(cudaFree(W->param_slab));
             W->param_slab = nullptr;
@@ -418,22 +417,11 @@ cudaError_t solve_device(const CplbParams& P, int im_kernel, const CplbInstParam
             base += align_up(doubles * sizeof(double));
             return p;
         };
-        const double** one[CPLB_NUM_INST_ARRAYS] = {&Q_one.mass, &Q_one.wrench, &Q_one.mu, &Q_one.F_thr, &Q_one.ground_z, &Q_one.com_ref, &Q_one.W_com,
-                                                     &Q_one.p_ref, &Q_one.F_ref, &Q_one.W_p, &Q_one.W_F};
-        const double** fd[CPLB_NUM_INST_ARRAYS] = {&Q_fd.mass, &Q_fd.wrench, &Q_fd.mu, &Q_fd.F_thr, &Q_fd.ground_z, &Q_fd.com_ref, &Q_fd.W_com,
-                                                    &Q_fd.p_ref, &Q_fd.F_ref, &Q_fd.W_p, &Q_fd.W_F};
-        const double** ls[CPLB_NUM_INST_ARRAYS] = {&Q_ls.mass, &Q_ls.wrench, &Q_ls.mu, &Q_ls.F_thr, &Q_ls.ground_z, &Q_ls.com_ref, &Q_ls.W_com,
-                                                    &Q_ls.p_ref, &Q_ls.F_ref, &Q_ls.W_p, &Q_ls.W_F};
         for (int a = 0; a < CPLB_NUM_INST_ARRAYS; a++) {
-            G.src[a] = src[a];
-            G.len[a] = len[a];
-            if (!src[a]) continue;
-            G.one[a] = carve((size_t)N * len[a]);
-            G.fd[a] = carve((size_t)N * G.reps_fd * len[a]);
-            G.ls[a] = carve((size_t)N * G.reps_ls * len[a]);
-            *one[a] = G.one[a];
-            *fd[a] = G.fd[a];
-            *ls[a] = G.ls[a];
+            if (!G.src[a]) continue;
+            Q_one.arr[a] = G.one[a] = carve((size_t)N * G.len[a]);
+            Q_fd.arr[a] = G.fd[a] = carve((size_t)N * G.reps_fd * G.len[a]);
+            Q_ls.arr[a] = G.ls[a] = carve((size_t)N * G.reps_ls * G.len[a]);
         }
     }
     DeviceEngine E{P, im_kernel, A, N, st, W, x0, x_out, lam_out, smem, smem_small, tail_limit, per_instance, G, Q_one, Q_fd, Q_ls};

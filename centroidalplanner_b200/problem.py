@@ -432,9 +432,7 @@ class BatchedCplProblem:
         layout: (N,) / (N, len) instance-major, (len, N) component-major.  on_device: x's torch device, or None (host)."""
         if not per_instance:
             return None, []
-        lens = {"mass": 1, "wrench": 6, "mu": 1, "force_threshold": len(self._names), "ground_z": 1, "com_ref": 3, "com_weight": 1,
-                "pos_ref": 3 * len(self._names), "force_ref": 3 * len(self._names), "pos_weight": len(self._names),
-                "force_weight": len(self._names)}
+        lens = {name: fixed + per_contact * len(self._names) for name, fixed, per_contact in _cabi.INSTANCE_PARAMS}
         st, keep = _cabi.InstanceParams(), []
         for name, arr in per_instance.items():
             if name not in lens:

@@ -7,7 +7,7 @@ import os
 import numpy as np
 
 import centroidalplanner_b200 as cpl
-from centroidalplanner_b200 import synthetic
+from centroidalplanner_b200 import _cabi, synthetic
 from oracle import cpl_oracle_py as orc
 
 RTOL = 1e-12  # north_star: "within 1e-12 relative (fp64)"
@@ -98,6 +98,26 @@ def configure(problem, env, names, env_name, rich=True, extra=None):
             problem.SetForceRef(nm, [1.0 + k, 2.0 - k, 100.0 + 10.0 * k])
             problem.SetContactPosWeight(nm, 0.5 + 0.25 * k)
             problem.SetContactForceWeight(nm, 0.001 * (k + 1))
+
+
+def set_oracle_instance(o, per_instance, i):
+    """Give oracle `o` the parameters of instance i of a per-instance dict (keys: _cabi.INSTANCE_PARAMS names, instance-major
+    NumPy arrays): the oracle then plays that instance's CplProblem."""
+    shared = {"mass": o.set_mass, "wrench": o.set_wrench, "mu": o.set_mu, "ground_z": o.set_ground_z, "com_ref": o.set_com_ref,
+              "com_weight": o.set_com_weight}
+    per_contact = {"force_threshold": o.set_force_threshold, "pos_ref": o.set_pos_ref, "force_ref": o.set_force_ref,
+                   "pos_weight": o.set_contact_pos_weight, "force_weight": o.set_contact_force_weight}
+    stride = {name: per for name, _, per in _cabi.INSTANCE_PARAMS}
+    for name, arr in per_instance.items():
+        row = arr[i]
+        if name in shared:
+            shared[name](row)
+        elif name in per_contact:
+            s = stride[name]
+            for k, nm in enumerate(o.names):
+                per_contact[name](nm, row[k] if s == 1 else row[s * k:s * k + s])
+        else:
+            raise ValueError(f"set_oracle_instance does not handle per-instance parameter '{name}'")
 
 
 def make_pair(case, mass=100.0, rich=True):

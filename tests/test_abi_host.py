@@ -29,6 +29,23 @@ def test_library_exports_every_symbol_the_header_declares():
     assert _cabi.load().cplb_abi_version() == 3
 
 
+def test_instance_params_table_matches_the_header():
+    """_cabi.INSTANCE_PARAMS (the ctypes struct and the length checks of the Python API) against cplb_instance_params in
+    include/cpl_batched.h: the member names in order, and the per-instance length each member's comment states."""
+    hdr = open(os.path.join(ROOT, "include", "cpl_batched.h")).read()
+    body = re.search(r"typedef struct cplb_instance_params \{(.*?)\} cplb_instance_params;", hdr, flags=re.S).group(1)
+    members = re.findall(r"const double \*(\w+);\s*/\*\s*(\S+)", body)
+    assert len(members) == len(re.findall(r";", body))
+
+    def length(text):  # "6" -> (6, 0), "nc" -> (0, 1), "3*nc" -> (0, 3)
+        m = re.fullmatch(r"(\d+)|(?:(\d+)\*)?nc", text)
+        assert m, text
+        return (int(m.group(1)), 0) if m.group(1) else (0, int(m.group(2) or 1))
+
+    assert tuple((name, *length(text)) for name, text in members) == _cabi.INSTANCE_PARAMS
+    assert [f[0] for f in _cabi.InstanceParams._fields_] == [name for name, _ in members]
+
+
 def test_product_never_imports_the_oracle():
     pkg = os.path.join(ROOT, "centroidalplanner_b200")
     for dirpath, _, files in os.walk(pkg):

@@ -19,7 +19,7 @@ import torch
 
 import centroidalplanner_b200 as cpl
 from centroidalplanner_b200 import _cabi, synthetic
-from helpers import configure, make_pair
+from helpers import configure, make_pair, set_oracle_instance
 from oracle import cpl_oracle_py as orc
 from test_gpu_solver_replay import CASES, oracle_side, product_side, same_bits
 from test_solve import starts
@@ -155,20 +155,8 @@ def test_per_instance_arrays_against_one_oracle_per_instance(cuda_device):
     xs = x0.cpu().numpy()
     rows = []
     for i in range(N):
-        op = oracle_side(case)
-        o = op.o
-        o.set_mass(arrs["mass"][i])
-        o.set_wrench(arrs["wrench"][i])
-        o.set_mu(arrs["mu"][i])
-        o.set_ground_z(arrs["ground_z"][i])
-        o.set_com_ref(arrs["com_ref"][i])
-        o.set_com_weight(arrs["com_weight"][i])
-        for k, nm in enumerate(names):
-            o.set_force_threshold(nm, arrs["force_threshold"][i, k])
-            o.set_pos_ref(nm, arrs["pos_ref"][i, 3 * k:3 * k + 3])
-            o.set_force_ref(nm, arrs["force_ref"][i, 3 * k:3 * k + 3])
-            o.set_contact_pos_weight(nm, arrs["pos_weight"][i, k])
-            o.set_contact_force_weight(nm, arrs["force_weight"][i, k])
+        o = oracle_side(case).o
+        set_oracle_instance(o, arrs, i)
         rows.append(replay(o, xs[i:i + 1]))
     want = {k: np.concatenate([r[k] for r in rows]) for k in KEYS}
     assert_same(got, want, "per-instance")

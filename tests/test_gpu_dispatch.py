@@ -17,7 +17,7 @@ import centroidalplanner_b200 as cpl
 from centroidalplanner_b200 import _cabi
 
 from helpers import CASES as ALL_CASES
-from helpers import assert_parity, make_pair
+from helpers import assert_parity, make_pair, set_oracle_instance
 
 pytestmark = pytest.mark.gpu
 
@@ -235,19 +235,7 @@ def test_instance_major_kernels_per_instance_parameters(case, kernel, cuda_devic
         pi["ground_z"] = rng.uniform(-0.2, 0.4, N)
     want = {"g": np.zeros((N, o.m)), "jac": np.zeros((N, o.nnz)), "cost": np.zeros(N), "grad": np.zeros((N, o.n))}
     for i in range(N):
-        o.set_mass(pi["mass"][i])
-        o.set_wrench(pi["wrench"][i])
-        o.set_mu(pi["mu"][i])
-        o.set_com_ref(pi["com_ref"][i])
-        o.set_com_weight(pi["com_weight"][i])
-        if "ground_z" in pi:
-            o.set_ground_z(pi["ground_z"][i])
-        for kk, nm in enumerate(o.names):
-            o.set_force_threshold(nm, pi["force_threshold"][i, kk])
-            o.set_pos_ref(nm, pi["pos_ref"][i, 3 * kk:3 * kk + 3])
-            o.set_force_ref(nm, pi["force_ref"][i, 3 * kk:3 * kk + 3])
-            o.set_contact_pos_weight(nm, pi["pos_weight"][i, kk])
-            o.set_contact_force_weight(nm, pi["force_weight"][i, kk])
+        set_oracle_instance(o, pi, i)
         e = o.eval(x[i])
         for key in want:
             want[key][i] = e[key]

@@ -6,7 +6,7 @@ import pytest
 import centroidalplanner_b200 as cpl
 from centroidalplanner_b200 import synthetic
 
-from helpers import CASES, assert_parity, make_pair, same_bits, to_instance_major
+from helpers import CASES, assert_parity, make_pair, same_bits, set_oracle_instance, to_instance_major
 
 pytestmark = pytest.mark.gpu
 
@@ -325,21 +325,8 @@ def test_per_instance_parameters(case, layout, path, cuda_device):
     if case.startswith("ground"):
         pi["ground_z"] = rng.uniform(-0.2, 0.4, N)
     want = {"g": np.zeros((N, o.m)), "jac": np.zeros((N, o.nnz)), "cost": np.zeros(N), "grad": np.zeros((N, o.n))}
-    names = o.names
     for i in range(N):
-        o.set_mass(pi["mass"][i])
-        o.set_wrench(pi["wrench"][i])
-        o.set_mu(pi["mu"][i])
-        o.set_com_ref(pi["com_ref"][i])
-        o.set_com_weight(pi["com_weight"][i])
-        if "ground_z" in pi:
-            o.set_ground_z(pi["ground_z"][i])
-        for k, nm in enumerate(names):
-            o.set_force_threshold(nm, pi["force_threshold"][i, k])
-            o.set_pos_ref(nm, pi["pos_ref"][i, 3 * k:3 * k + 3])
-            o.set_force_ref(nm, pi["force_ref"][i, 3 * k:3 * k + 3])
-            o.set_contact_pos_weight(nm, pi["pos_weight"][i, k])
-            o.set_contact_force_weight(nm, pi["force_weight"][i, k])
+        set_oracle_instance(o, pi, i)
         e = o.eval(x[i])
         for key in want:
             want[key][i] = e[key]
@@ -385,12 +372,7 @@ def test_per_instance_constraint_only_evaluations(case, N, want, misaligned, cud
           "force_threshold": rng.uniform(0, 30, (N, nc)), "ground_z": rng.uniform(-0.2, 0.4, N)}
     ref = {"g": np.zeros((N, o.m)), "jac": np.zeros((N, o.nnz))}
     for i in range(N):
-        o.set_mass(pi["mass"][i])
-        o.set_wrench(pi["wrench"][i])
-        o.set_mu(pi["mu"][i])
-        o.set_ground_z(pi["ground_z"][i])
-        for k, nm in enumerate(o.names):
-            o.set_force_threshold(nm, pi["force_threshold"][i, k])
+        set_oracle_instance(o, pi, i)
         e = o.eval(x[i], want=("g", "jac"))
         ref["g"][i], ref["jac"][i] = e["g"], e["jac"]
 
