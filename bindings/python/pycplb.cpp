@@ -182,6 +182,16 @@ PYBIND11_MODULE(pycplb, m)
         }, py::arg("num_instances"), py::arg("x"), py::arg("num_wrong") = 0, py::arg("num_wrong_outside") = 0, py::arg("max_rel_error") = 0,
              py::arg("worst_row") = 0, py::arg("worst_col") = 0, py::arg("jac_fd") = 0, py::arg("grad_fd") = 0, py::arg("stream") = 0,
              py::arg("perturbation") = 1e-8, py::arg("tol") = 1e-4)
+        // Jacobian products at x (cplb_jacobian_products_device); raw device pointers, instance-major (0 = NULL)
+        .def("jacobian_products_device", [](cplb::BatchedProblem& p, int64_t N, uintptr_t x, uintptr_t lam, uintptr_t obj_factor, uintptr_t x_bar,
+                                            uintptr_t v, uintptr_t g_dot, uintptr_t f_dot, uintptr_t stream) {
+            const cplb_jacobian_products_args a{N, reinterpret_cast<const double*>(x), nullptr, reinterpret_cast<const double*>(lam),
+                                                reinterpret_cast<const double*>(obj_factor), reinterpret_cast<double*>(x_bar),
+                                                reinterpret_cast<const double*>(v), reinterpret_cast<double*>(g_dot), reinterpret_cast<double*>(f_dot)};
+            py::gil_scoped_release nogil;
+            p.JacobianProductsDevice(a, reinterpret_cast<void*>(stream));
+        }, py::arg("num_instances"), py::arg("x"), py::arg("lam") = 0, py::arg("obj_factor") = 0, py::arg("x_bar") = 0, py::arg("v") = 0,
+             py::arg("g_dot") = 0, py::arg("f_dot") = 0, py::arg("stream") = 0)
         // raw device pointers (e.g. torch.Tensor.data_ptr()), either layout, asynchronous on `stream`
         .def("eval_device", [](cplb::BatchedProblem& p, int64_t N, int layout, int64_t ld, uintptr_t x, uintptr_t g, uintptr_t jac,
                                uintptr_t cost, uintptr_t grad, uintptr_t stream) {

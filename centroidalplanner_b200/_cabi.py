@@ -79,6 +79,12 @@ class DerivativeTestOutputs(C.Structure):
                 ("worst_col", C.c_void_p), ("jac_fd", C.c_void_p), ("grad_fd", C.c_void_p)]
 
 
+class JacobianProductsArgs(C.Structure):
+    """cplb_jacobian_products_args (device pointers; None = NULL)"""
+    _fields_ = [("num_instances", C.c_int64), ("x", C.c_void_p), ("per_instance", C.POINTER(InstanceParams)), ("lambda_", C.c_void_p),
+                ("obj_factor", C.c_void_p), ("x_bar", C.c_void_p), ("v", C.c_void_p), ("g_dot", C.c_void_p), ("f_dot", C.c_void_p)]
+
+
 # name -> (restype, argtypes); every symbol include/cpl_batched.h declares
 PROTOTYPES = {
     "cplb_create": (C.c_int, [C.c_int32, C.POINTER(C.c_char_p), C.c_int, C.c_double, C.c_int32, C.POINTER(C.c_void_p)]),
@@ -140,6 +146,7 @@ PROTOTYPES = {
     "cplb_derivative_test_default_options": (None, [C.POINTER(DerivativeTestOptions)]),
     "cplb_derivative_test_device": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.POINTER(InstanceParams), C.POINTER(DerivativeTestOptions),
                                               C.POINTER(DerivativeTestOutputs), C.c_void_p]),
+    "cplb_jacobian_products_device": (C.c_int, [C.c_void_p, C.POINTER(JacobianProductsArgs), C.c_void_p]),
     "cplb_host_alloc": (C.c_int, [C.c_size_t, C.POINTER(C.c_void_p)]),
     "cplb_host_free": (C.c_int, [C.c_void_p]),
     "cplb_set_component_major_kernel": (C.c_int, [C.c_void_p, C.c_int32]),

@@ -476,6 +476,10 @@ public:
         check(cplb_derivative_test_device(_p, N, x, per_instance, options, &out, stream));
     }
 
+    // Products with the Jacobian at x without materialising it (cplb_jacobian_products_device): x_bar = obj_factor * grad f +
+    // J^T lambda and/or g_dot = J v, f_dot = grad f . v.  Device pointers in `args`; asynchronous on `stream`.
+    void JacobianProductsDevice(const cplb_jacobian_products_args& args, void* stream) { check(cplb_jacobian_products_device(_p, &args, stream)); }
+
 private:
     std::vector<std::string> _contact_names;
     env::EnvironmentClass::Ptr _env;

@@ -21,6 +21,7 @@
 #include "cplb_kernels.h"
 #include "cplb_layout.hpp"
 #include "cplb_params.h"
+#include "cplb_products.h"
 #include "cplb_solver.h"
 
 namespace {
@@ -1510,6 +1511,36 @@ cplb_status cplb_derivative_test_device(cplb_problem* p, int64_t num_instances, 
     cudaError_t e = cplb::launch_derivative_test(p->P, per_inst ? &q : nullptr, x, num_instances, p->slot_of, o.perturbation, o.tol, dout,
                                                  static_cast<cudaStream_t>(cuda_stream));
     if (e != cudaSuccess) return cuda_fail(e, "cplb_derivative_test_device");
+    p->launches.fetch_add(1, std::memory_order_relaxed);
+    return CPLB_OK;
+}
+
+// ---- Jacobian products ---------------------------------------------------------------------------------------------------------
+
+cplb_status cplb_jacobian_products_device(cplb_problem* p, const cplb_jacobian_products_args* args, void* cuda_stream)
+{
+    CPLB_REQUIRE(p);
+    CPLB_REQUIRE(args);
+    const cplb_jacobian_products_args& a = *args;
+    if (a.num_instances < 0) return fail(CPLB_INVALID_ARGUMENT, "num_instances is negative");
+    if (a.num_instances > 0 && a.x == nullptr) return fail(CPLB_NULL_POINTER, "x is NULL");
+    if (a.x_bar && !a.lambda && !a.obj_factor)
+        return fail(CPLB_INVALID_ARGUMENT, "x_bar is requested but lambda and obj_factor are both NULL: the reverse product has no term");
+    if ((a.g_dot || a.f_dot) && a.v == nullptr) return fail(CPLB_NULL_POINTER, "v is NULL but g_dot or f_dot is requested");
+    if (!a.x_bar && !a.g_dot && !a.f_dot) return fail(CPLB_INVALID_ARGUMENT, "no output requested: set x_bar, g_dot or f_dot");
+    if (p->pipes.size() > 1)
+        return fail(CPLB_INVALID_ARGUMENT, "cplb_jacobian_products_device needs a single-device problem (one batch per GPU)");
+    if (a.num_instances > INT32_MAX) return fail(CPLB_INVALID_ARGUMENT, "num_instances (%lld) must be below 2^31", (long long)a.num_instances);
+    if (a.num_instances == 0) return CPLB_OK;
+    cplb_status st = bind_device(p);
+    if (st != CPLB_OK) return st;
+    DeviceGuard dg(p->device);
+    if (!dg.ok) return fail(CPLB_CUDA_ERROR, "cudaSetDevice(%d) failed", p->device);
+    CplbInstParams q;
+    const bool per_inst = instance_arrays(a.per_instance, &q);
+    const cplb::ProductArgs pa{a.x, a.lambda, a.obj_factor, a.x_bar, a.v, a.g_dot, a.f_dot, a.num_instances};
+    cudaError_t e = cplb::launch_jacobian_products(p->P, per_inst ? &q : nullptr, pa, static_cast<cudaStream_t>(cuda_stream));
+    if (e != cudaSuccess) return cuda_fail(e, "cplb_jacobian_products_device");
     p->launches.fetch_add(1, std::memory_order_relaxed);
     return CPLB_OK;
 }

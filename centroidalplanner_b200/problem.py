@@ -620,6 +620,49 @@ class BatchedCplProblem:
         del keep
         return rep
 
+    def JacobianProducts(self, x, lam=None, obj_factor=None, v=None, per_instance=None, stream=None):
+        """Products with the Jacobian at x without materialising it (cplb_jacobian_products_device), for N instances at once:
+        reverse  x_bar = obj_factor * grad f(x) + J(x)^T lam   (when lam or obj_factor is given)
+        forward  g_dot = J(x) v,  f_dot = grad f(x) . v        (when v is given)
+        x (N, n), lam (N, m), obj_factor (N,), v (N, n): contiguous float64 CUDA tensors on one device.  The results are bit for bit
+        those of multiplying eval()'s Jacobian and gradient in slot order (include/cpl_batched.h).  Asynchronous on the current
+        stream (or `stream`); per_instance: dict of per-instance parameter arrays as for eval().  Returns a dict with the requested
+        subset of 'x_bar' (N, n), 'g_dot' (N, m) and 'f_dot' (N,)."""
+        import torch
+
+        if not (_is_torch(x) and x.is_cuda):
+            raise ValueError("JacobianProducts needs x as a CUDA tensor (there is no CPU evaluation path)")
+        N, dev = x.shape[0], x.device
+        for name, t, shape in (("x", x, (N, self.n)), ("lam", lam, (N, self.m)), ("obj_factor", obj_factor, (N,)), ("v", v, (N, self.n))):
+            if t is None:
+                continue
+            if not (_is_torch(t) and t.is_cuda and t.dtype == torch.float64 and t.is_contiguous()):
+                raise ValueError(f"{name} must be a contiguous float64 CUDA tensor")
+            if t.device != dev:
+                raise ValueError(f"{name} lives on {t.device}, x on {dev}")
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {shape}")
+        if lam is None and obj_factor is None and v is None:
+            raise ValueError("JacobianProducts needs lam and/or obj_factor (reverse product) or v (forward product)")
+        bound = self.GetDevice()
+        if bound >= 0 and bound != dev.index:
+            raise ValueError(f"this problem evaluates on cuda:{bound}; x lives on {dev}")
+        res = {}
+        if lam is not None or obj_factor is not None:
+            res["x_bar"] = torch.empty(N, self.n, dtype=torch.float64, device=dev)
+        if v is not None:
+            res["g_dot"] = torch.empty(N, self.m, dtype=torch.float64, device=dev)
+            res["f_dot"] = torch.empty(N, dtype=torch.float64, device=dev)
+        pi, keep = self._instance_params(per_instance, N, _cabi.INSTANCE_MAJOR, dev)
+        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        args = _cabi.JacobianProductsArgs(N, x.data_ptr(), None if pi is None else C.pointer(pi), ptr(lam), ptr(obj_factor), ptr(res.get("x_bar")),
+                                          ptr(v), ptr(res.get("g_dot")), ptr(res.get("f_dot")))
+        s = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
+        with torch.cuda.device(dev):
+            _check(self._lib.cplb_jacobian_products_device(self._h, C.byref(args), C.c_void_p(s)))
+        del keep
+        return res
+
     # the four ifopt::Problem entry points IpoptAdapter calls, batched
     def EvaluateConstraints(self, x, **kw):
         return self.eval(x, g=True, jac=False, **kw)["g"]

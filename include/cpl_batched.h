@@ -429,6 +429,43 @@ cplb_status cplb_derivative_test_device(cplb_problem *p, int64_t num_instances, 
                                         const cplb_derivative_test_options *options, const cplb_derivative_test_outputs *out,
                                         void *cuda_stream);
 
+/* ---- Jacobian products ------------------------------------------------------------------------------------------------------ */
+
+/* What a first-order or penalty method, the Lagrangian gradient of an outside solver, or a reverse-mode autodiff caller needs
+ * from the Jacobian, without materialising it: one kernel reads x (and lambda / v) and writes the products (csrc/cplb_products.cu).
+ *   reverse  x_bar = obj_factor * grad f(x) + J(x)^T lambda        (IPOPT's sigma / lambda naming, as in eval_h)
+ *   forward  g_dot = J(x) v,   f_dot = grad f(x) . v
+ * Bit contract: the results are exactly those of a caller that materialises J and the gradient with cplb_eval_device (the
+ * evaluator's bits, every structural slot present, Ground's explicit zeros included) and multiplies them in slot order, with one
+ * IEEE multiply and one IEEE add per term and no FMA:
+ *   x_bar[c] starts at obj_factor * grad[c] (at +0.0 when obj_factor is NULL); then + J[s] * lambda[iRow[s]] for every structural
+ *            slot s with jCol[s] == c, slots ascending (= rows ascending);
+ *   g_dot[r] starts at +0.0; then + J[s] * v[jCol[s]] for the slots of row r, slots ascending (= columns ascending);
+ *   f_dot    starts at +0.0; then + grad[c] * v[c] for c = 0..n-1.
+ * So 0 * Inf in a structural-zero slot gives NaN, as it would for the materialising caller.  (A multiply is dropped only where the
+ * result has the same bits: by the 1.0 identity entries.) */
+typedef struct cplb_jacobian_products_args {
+    int64_t num_instances;
+    const double *x;                          /* [N n] instance-major, DEVICE */
+    const cplb_instance_params *per_instance; /* NULL, or device arrays as for cplb_solve_device (instance-major) */
+    /* reverse mode */
+    const double *lambda;                     /* [N m] or NULL (no J^T term) */
+    const double *obj_factor;                 /* [N]   or NULL (no gradient term) */
+    double *x_bar;                            /* [N n] or NULL (reverse product not computed) */
+    /* forward mode */
+    const double *v;                          /* [N n] */
+    double *g_dot;                            /* [N m] or NULL */
+    double *f_dot;                            /* [N]   or NULL */
+} cplb_jacobian_products_args;
+
+/* Every array is a DEVICE array on the problem's device, instance-major.  Asynchronous on `cuda_stream`; one launch, counted in
+ * cplb_get_launch_count.  Argument errors are reported before any CUDA call: NULL p or args, or NULL x with N > 0 ->
+ * CPLB_NULL_POINTER; g_dot or f_dot set with v NULL -> CPLB_NULL_POINTER; x_bar set with both lambda and obj_factor NULL, no output
+ * requested, N < 0 or N >= 2^31 -> CPLB_INVALID_ARGUMENT.  N = 0 -> CPLB_OK, nothing launched.  Single-device problems only, like
+ * cplb_solve_device.  Every shape up to CPLB_MAX_CONTACTS contacts is supported, in every environment.  No derivatives with
+ * respect to the parameters, no second derivatives. */
+cplb_status cplb_jacobian_products_device(cplb_problem *p, const cplb_jacobian_products_args *args, void *cuda_stream);
+
 /* Pinned host memory for cplb_eval_host buffers (cudaHostAlloc / cudaFreeHost). */
 cplb_status cplb_host_alloc(size_t bytes, void **out);
 cplb_status cplb_host_free(void *ptr);
