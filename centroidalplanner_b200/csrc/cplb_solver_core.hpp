@@ -616,8 +616,13 @@ CPLB_HD void phase_round_begin(const Team& team, const Shape& S, const State& T,
         }
       if (team.rank == 0) {
         // IPOPT's test (scaled error <= tol, unscaled violation <= constr_viol_tol) switches the instance to the feasibility
-        // polish; it is done when the constraints hold to polish_viol_tol as well
+        // polish; it is done when the constraints hold to polish_viol_tol as well.  The polish moves x with the multipliers
+        // frozen, so the test must still hold where it ends: a polished iterate that lost it (the scaled error grew past tol)
+        // leaves the polish and takes Newton steps again, undamped (the polish's line searches raise the Levenberg-Marquardt
+        // damping; kept, it stalls the Newton steps of a degenerate problem) -- SUCCEEDED always means E0 <= tol at the returned
+        // iterate.
         if (E0 <= O.tol && vmax <= O.constr_viol_tol) T.polish[i] = 1;
+        else if (T.polish[i] && vmax <= O.polish_viol_tol) { T.polish[i] = 0; T.delta_lm[i] = 0.0; }
         if (T.polish[i] && vmax <= O.polish_viol_tol) T.status[i] = kSuccess;
         else if (!finite_d(E0)) T.status[i] = kInvalidNumber;
         T.out_dual[i] = dual;

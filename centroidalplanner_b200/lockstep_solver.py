@@ -290,8 +290,13 @@ class LockStepInteriorPoint:
             viol = (torch.clamp(sl - c, min=0) + torch.clamp(c - su, min=0)) / dc                           # unscaled row violation (relaxed bounds)
             vmax = viol.amax(1)
             # IPOPT's test (scaled error <= tol, unscaled violation <= constr_viol_tol) switches an instance to the
-            # feasibility polish; it is done when the constraints hold to polish_viol_tol as well
-            polish = polish | ((status < 0) & (E0 <= self.tol) & (vmax <= self.constr_viol_tol))
+            # feasibility polish; it is done when the constraints hold to polish_viol_tol as well -- and the test still holds there:
+            # a polished iterate whose scaled error grew past tol (the polish moves x with the multipliers frozen) leaves the
+            # polish and takes Newton steps again (csrc/cplb_solver_core.hpp, phase_round_begin)
+            converged = (status < 0) & (E0 <= self.tol) & (vmax <= self.constr_viol_tol)
+            unpolish = ~converged & polish & (vmax <= self.polish_viol_tol)     # ... and its Newton steps start undamped
+            delta_lm = torch.where(unpolish, torch.zeros_like(delta_lm), delta_lm)
+            polish = polish & ~unpolish | converged
             done_now = (status < 0) & polish & (vmax <= self.polish_viol_tol)
             status = torch.where(done_now, torch.full_like(status, SUCCESS), status)
             nonfinite = (status < 0) & ~(torch.isfinite(E0))

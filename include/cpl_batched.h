@@ -355,7 +355,10 @@ typedef struct cplb_solver_options {
 } cplb_solver_options;
 void cplb_solver_default_options(cplb_solver_options *options);
 
-#define CPLB_SOLVE_SUCCEEDED 0              /* Ipopt::Solve_Succeeded */
+#define CPLB_SOLVE_SUCCEEDED 0              /* Ipopt::Solve_Succeeded: at the final iterate the scaled error (dual_inf, the
+                                               complementarity, the scaled primal residual) is <= tol and constr_viol <=
+                                               polish_viol_tol.  (A feasibility polish with frozen multipliers follows IPOPT's
+                                               test; an iterate it leaves with a scaled error above tol takes Newton steps again.) */
 #define CPLB_SOLVE_MAX_ITERATIONS 1         /* Ipopt::Maximum_Iterations_Exceeded */
 #define CPLB_SOLVE_INVALID_NUMBER 2         /* Ipopt::Invalid_Number_Detected */
 
@@ -365,11 +368,17 @@ typedef struct cplb_solve_outputs {
                              reads one instance's slice (cplb::BatchedProblem::GetSolution) */
     int32_t *status;      /* [N]    CPLB_SOLVE_* */
     int32_t *iterations;  /* [N] */
-    double *cost;         /* [N]    MinimizeCentroidalVariables::GetCost at x */
-    double *constr_viol;  /* [N]    max violation of the constraint bounds at x; NaN for a start rejected as
-                             CPLB_SOLVE_INVALID_NUMBER before its first iteration (0 iterations) */
-    double *dual_inf;     /* [N]    scaled dual infeasibility at x; NaN for such a rejected start */
-    double *lam;          /* [N m]  constraint multipliers, or NULL */
+    double *cost;         /* [N]    MinimizeCentroidalVariables::GetCost at the final iterate.  That is x, unless the clipping moved an
+                             entry of x back onto its bound (by at most bound_relax_factor * max(|bound|, 1)): cost, constr_viol
+                             and dual_inf are the values of the iterate before the clipping */
+    double *constr_viol;  /* [N]    max over rows of the violation of the row's bounds at the final iterate: equality rows against
+                             their value, inequality rows against their bounds relaxed by bound_relax_factor * max(|bound|, 1)
+                             (the bounds the solver works with); NaN for a start rejected as CPLB_SOLVE_INVALID_NUMBER before its
+                             first iteration (0 iterations) */
+    double *dual_inf;     /* [N]    scaled dual infeasibility (IPOPT's, divided by s_d) at the final iterate; NaN for such a
+                             rejected start */
+    double *lam;          /* [N m]  constraint multipliers, unscaled, IPOPT's sign (L = f + lam^T g: >= 0 on an active upper
+                             bound, <= 0 on an active lower one), or NULL */
     int32_t *rounds;              /* HOST: lock-step rounds executed, or NULL */
     int64_t *evaluations;         /* HOST: batched evaluations launched, or NULL */
     int64_t *instance_evaluations; /* HOST: instances evaluated in total, or NULL */

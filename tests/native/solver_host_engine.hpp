@@ -6,6 +6,7 @@
 
 #include <cmath>
 #include <cstdio>
+#include <thread>
 #include <utility>
 #include <vector>
 
@@ -17,6 +18,10 @@ namespace solver {
 
 struct HostEngine {
     cpl_oracle* o;
+    // one oracle per instance (a sweep in which every instance is its own planning problem), or empty: o evaluates every point.
+    // An evaluated row goes to the oracle of the instance whose slot it belongs to (list_cur: before the first round the slots
+    // are the instances), like the per-instance parameter rows the GPU gathers into slot order.
+    std::vector<cpl_oracle*> per;
     ShapeHost SH;
     Shape S;
     State T{};
@@ -99,13 +104,14 @@ struct HostEngine {
     long long tail(long long running, int it0)
     {
         long long rounds = 0;
-        auto eval = [&](const double* x, int count, unsigned flags, double* g, double* jac, double* cost, double* grad) {
-            (void)flags;
-            for (int a = 0; a < count; a++)
-                cpl_oracle_eval(o, x + (long long)a * S.n, g ? g + (long long)a * S.m : nullptr, jac ? jac + (long long)a * S.nnz : nullptr,
-                                cost ? cost + a : nullptr, grad ? grad + (long long)a * S.n : nullptr);
-        };
         for (long long b = 0; b < running; b++) {
+            const cpl_oracle* ob = per.empty() ? o : per[T.list_cur[b]];
+            auto eval = [&](const double* x, int count, unsigned flags, double* g, double* jac, double* cost, double* grad) {
+                (void)flags;
+                for (int a = 0; a < count; a++)
+                    cpl_oracle_eval(ob, x + (long long)a * S.n, g ? g + (long long)a * S.m : nullptr, jac ? jac + (long long)a * S.nnz : nullptr,
+                                    cost ? cost + a : nullptr, grad ? grad + (long long)a * S.n : nullptr);
+            };
             for (int it = it0;;) {
                 tail_iteration(team, S, T, O, b, q, eval);
                 rounds++;
@@ -118,10 +124,28 @@ struct HostEngine {
         return rounds;
     }
     void finish() { for (long long i = 0; i < N; i++) phase_finish(team, S, T, i, x_out.data(), lam_out.data()); }
-    void eval_full(long long cnt) { cpl_oracle_eval_batch(o, cnt, T.xc, T.ev_c, T.ev_jv, T.ev_f, T.ev_df, threads); }
-    void eval_fd(long long cnt) { cpl_oracle_eval_batch(o, cnt * (S.nf + 1), T.x_fd, nullptr, T.jac_fd, nullptr, T.grad_fd, threads); }
-    void eval_ls(long long cnt) { cpl_oracle_eval_batch(o, cnt * kCandidates, T.x_ls, T.g_ls, nullptr, T.cost_ls, nullptr, threads); }
-    void eval_soc(long long cnt) { cpl_oracle_eval_batch(o, cnt, T.x_soc, T.g_soc, nullptr, T.cost_soc, nullptr, threads); }
+    // `rows` points, `width` consecutive rows per slot
+    void eval_rows(long long rows, long long width, const double* X, double* g, double* jac, double* cost, double* grad)
+    {
+        if (per.empty()) {
+            cpl_oracle_eval_batch(o, rows, X, g, jac, cost, grad, threads);
+            return;
+        }
+        auto part = [&](long long r0, long long r1) {
+            for (long long r = r0; r < r1; r++)
+                cpl_oracle_eval(per[T.list_cur[r / width]], X + r * S.n, g ? g + r * S.m : nullptr, jac ? jac + r * S.nnz : nullptr,
+                                cost ? cost + r : nullptr, grad ? grad + r * S.n : nullptr);
+        };
+        const long long nt = threads < rows ? threads : rows, chunk = (rows + nt - 1) / nt;
+        std::vector<std::thread> pool;
+        for (long long t = 1; t < nt; t++) pool.emplace_back(part, t * chunk < rows ? t * chunk : rows, (t + 1) * chunk < rows ? (t + 1) * chunk : rows);
+        part(0, chunk < rows ? chunk : rows);
+        for (auto& th : pool) th.join();
+    }
+    void eval_full(long long cnt) { eval_rows(cnt, 1, T.xc, T.ev_c, T.ev_jv, T.ev_f, T.ev_df); }
+    void eval_fd(long long cnt) { eval_rows(cnt * (S.nf + 1), S.nf + 1, T.x_fd, nullptr, T.jac_fd, nullptr, T.grad_fd); }
+    void eval_ls(long long cnt) { eval_rows(cnt * kCandidates, kCandidates, T.x_ls, T.g_ls, nullptr, T.cost_ls, nullptr); }
+    void eval_soc(long long cnt) { eval_rows(cnt, 1, T.x_soc, T.g_soc, nullptr, T.cost_soc, nullptr); }
 };
 
 }  // namespace solver

@@ -1,7 +1,8 @@
 // C entry to the CPU replay of the native solve round (solver_host_engine.hpp), for tests/test_gpu_solver_replay.py: solves N
 // starts of the problem an oracle handle describes with the per-instance code of csrc/cplb_solver_core.hpp, one thread per
 // instance, the oracle behind the evaluations.  Link against the oracle/libcpl_oracle.so the ctypes wrapper loads, so that the
-// wrapper's handle (cpl_oracle_py.Oracle._h) is valid here.  TEST INFRASTRUCTURE.
+// wrapper's handle (cpl_oracle_py.Oracle._h) is valid here.  A second entry takes one oracle per instance (per-instance
+// parameter sweeps).  TEST INFRASTRUCTURE.
 #include <cstdint>
 #include <cstring>
 
@@ -12,10 +13,10 @@ using namespace cplb::solver;
 
 // stats (may be NULL): [rounds, evaluations, instance_evaluations, tail_instances].  tail_instances < 0 counts as 0 (lock-step
 // rounds to the end): the host has no GPU to fill, and where the tail takes over does not change any instance's result.
+// per (may be NULL): N oracle handles, per[i] the problem of instance i (same shape and bounds as o); o = per[0] then.
 // Returns 0, or -1 on bad arguments.
-extern "C" int cplb_replay_solve(cpl_oracle* o, int64_t N, const double* x0, const cplb_solver_options* opt, double* x, double* lam,
-                                 int32_t* status, int32_t* iterations, double* cost, double* constr_viol, double* dual_inf, int64_t* stats,
-                                 int threads)
+static int replay(cpl_oracle* o, cpl_oracle* const* per, int64_t N, const double* x0, const cplb_solver_options* opt, double* x, double* lam,
+                  int32_t* status, int32_t* iterations, double* cost, double* constr_viol, double* dual_inf, int64_t* stats, int threads)
 {
     if (!o || N <= 0 || !x0 || !opt || !x || !status || !iterations || !cost || !constr_viol || !dual_inf) return -1;
     int n, m, nnz;
@@ -28,6 +29,15 @@ extern "C" int cplb_replay_solve(cpl_oracle* o, int64_t N, const double* x0, con
 
     HostEngine E;
     E.o = o;
+    if (per) {
+        for (int64_t i = 0; i < N; i++) {
+            int ni, mi, nnzi;
+            if (!per[i]) return -1;
+            cpl_oracle_dims(per[i], &ni, &mi, &nnzi);
+            if (ni != n || mi != m || nnzi != nnz) return -1;
+        }
+        E.per.assign(per, per + N);
+    }
     E.N = N;
     E.threads = threads > 0 ? threads : 1;
     E.O = Options{opt->tol, opt->mu_init, opt->bound_push, opt->bound_frac, opt->nlp_scaling_max_gradient, opt->constr_viol_tol,
@@ -52,4 +62,21 @@ extern "C" int cplb_replay_solve(cpl_oracle* o, int64_t N, const double* x0, con
         stats[3] = st.tail_instances;
     }
     return 0;
+}
+
+extern "C" int cplb_replay_solve(cpl_oracle* o, int64_t N, const double* x0, const cplb_solver_options* opt, double* x, double* lam,
+                                 int32_t* status, int32_t* iterations, double* cost, double* constr_viol, double* dual_inf, int64_t* stats,
+                                 int threads)
+{
+    return replay(o, nullptr, N, x0, opt, x, lam, status, iterations, cost, constr_viol, dual_inf, stats, threads);
+}
+
+// The replay of a sweep: instance i solves the problem of oracle o[i] (its own cplb_instance_params, set on that oracle).  Every
+// evaluated point goes to the oracle of its instance; the variable / constraint bounds are o[0]'s (the bounds stay the problem's).
+extern "C" int cplb_replay_solve_per_instance(cpl_oracle* const* o, int64_t N, const double* x0, const cplb_solver_options* opt, double* x,
+                                              double* lam, int32_t* status, int32_t* iterations, double* cost, double* constr_viol,
+                                              double* dual_inf, int64_t* stats, int threads)
+{
+    if (!o || N <= 0) return -1;
+    return replay(o[0], o, N, x0, opt, x, lam, status, iterations, cost, constr_viol, dual_inf, stats, threads);
 }
